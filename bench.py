@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the log-posterior hot path (driver contract: one JSON line on stdout).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json config 3, the BSM fit the north star's roofline target names): the batched
 BSM dim-6 / texture-OET log-posterior -- 6 SM parameters + log10(Lambda) per point, 20 energy bins,
@@ -33,6 +33,11 @@ the hot path over that batch = ONE kernel launch.
 baseline/_ref (git-ignored, travels with the snapshot; `kind: "reference"`), else the oracle port
 (`kind: "port"`) -- on all host cores for the same metric and config: exactly K steps after W warm-up
 steps, each step a bounded sample of the workload.
+
+`--dump-outputs DIR` writes what the last of the K timed GPU steps computed, the log-posterior of the batch, as
+float64: DIR/lnprob.npy holds every point (32 MiB).  With N > 1 ranks, rank r writes DIR/lnprob_rank<r>.npy holding
+every N-th point of its batch (rows 0, N, 2N, ...), so the files total 32 MiB whatever N is.  theta is drawn from a
+fixed seed per rank, so two builds run with the same arguments can be compared output for output.
 """
 
 import argparse
@@ -319,7 +324,7 @@ def run_reference(opts):
         return
     import multiprocessing as mp
     cores = os.cpu_count() or 1
-    steps, warmup = max(1, opts.steps), max(0, opts.warmup)
+    steps, warmup = opts.steps, max(0, opts.warmup)
     per_core = int(min(150, max(4, round(30.0 * 90.0 / (steps + warmup)))))   # ~90 evals/s/core
     kind = 'reference' if _reference_problem() is not None else 'port'         # set up before the fork: workers inherit it
     if kind == 'port':
@@ -466,6 +471,9 @@ def run_gpu(opts):
     clock_info = clocks.stop() if rank == 0 else None
     value = world * n * opts.steps / (ms * 1e-3)
     kernel_ms = ms / opts.steps
+    if opts.dump_outputs:
+        name = 'lnprob.npy' if world == 1 else 'lnprob_rank%d.npy' % rank
+        np.save(os.path.join(opts.dump_outputs, name), out[::world].cpu().numpy())   # one world-th of each rank's rows
 
     # -- end to end through the host API
     out_host = torch.empty(n, dtype=torch.float64).pin_memory()
@@ -721,7 +729,14 @@ def main():
     ap.add_argument('--configs', type=int, default=1, help='1: also time the sampler-shaped configs C2/C3/C5 (secondary section)')
     ap.add_argument('--scan-mode', default='anarchic', choices=['unitary', 'x', 'texture', 'anarchic'])
     ap.add_argument('--sustain-s', type=float, default=1.2, help='length of the sustained k_lnprob loop after the K timed steps (0 = skip)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the log-posterior of the last timed step to DIR (GPU arm; 32 MiB in all)')
     opts = ap.parse_args()
+    if opts.steps < 1:
+        ap.error('--steps must be at least 1')
+    if opts.dump_outputs:
+        if opts.impl == 'reference':
+            ap.error('--dump-outputs writes the outputs of the GPU arm; the reference arm keeps none')
+        os.makedirs(opts.dump_outputs, exist_ok=True)
     opts.warmup = max(opts.warmup, 3) if opts.impl == 'b200' else opts.warmup
     if opts.impl == 'reference':
         run_reference(opts)

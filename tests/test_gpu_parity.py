@@ -1410,3 +1410,31 @@ def test_multi_gpu_nccl_scan_evidence_and_sweep_are_rank_count_invariant(torch):
                          text=True, timeout=900)
     assert res.returncode == 0, res.stdout[-3000:]
     assert res.stdout.count('bit-identical=True') == 3 and 'ok=True' in res.stdout and 'sweep=True' in res.stdout
+
+
+def test_bench_dumps_the_last_timed_step(torch, tmp_path):
+    """`bench.py --dump-outputs DIR`: after exactly K timed launches, DIR/lnprob.npy holds the float64 log-posterior of every
+    point of the seeded benchmark batch, in batch order -- the same values the public API computes for those rows -- and the
+    dump stays within its 64 MB budget."""
+    import json
+    import subprocess
+
+    import bench   # the repository root is on sys.path (conftest.py)
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    res = subprocess.run([sys.executable, os.path.join(root, 'bench.py'), '--steps', '2', '--warmup', '3', '--cpu-evals', '0',
+                          '--scan-samples', '0', '--configs', '0', '--sustain-s', '0', '--dump-outputs', str(tmp_path / 'out')],
+                         stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600)
+    assert res.returncode == 0, res.stderr[-3000:]
+    line = json.loads(res.stdout)
+    assert line['steps'] == 2 and line['gpu_launches'] == 2
+    assert sorted(os.listdir(tmp_path / 'out')) == ['lnprob.npy']
+    assert os.path.getsize(tmp_path / 'out' / 'lnprob.npy') <= 64 * 10 ** 6
+    got = np.load(tmp_path / 'out' / 'lnprob.npy')
+    n = bench.WALKERS * bench.CHAINS
+    assert got.dtype == np.float64 and got.shape == (n,)
+    (args, asimov, pset), models_ = bench.build_problem()
+    sel = np.sort(np.random.default_rng(0).choice(n, 4096, replace=False))
+    theta = bench.synth_theta(pset, n, 25, models_)[sel]
+    want = llh.LnProb(args, asimov, pset).evaluate(theta).cpu().numpy()
+    assert np.isfinite(want).mean() > 0.5
+    np.testing.assert_allclose(got[sel], want, rtol=1e-12, atol=0)

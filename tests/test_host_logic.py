@@ -603,6 +603,21 @@ def test_bench_reference_arm_prints_one_contract_line():
     assert gpu.returncode != 0 and 'no CUDA device' in (gpu.stderr + gpu.stdout)
 
 
+def test_bench_refuses_no_timed_steps_and_a_dump_of_the_reference_arm(tmp_path):
+    """`--steps` is the number of timed steps, so 0 is refused rather than rounded up; `--dump-outputs` belongs to the GPU
+    arm (the reference arm keeps no outputs) and is refused before any work or any file is written."""
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES='')
+    for extra in (['--steps', '0'], ['--impl', 'reference', '--steps', '0'],
+                  ['--impl', 'reference', '--dump-outputs', str(tmp_path / 'out')]):
+        res = subprocess.run([sys.executable, os.path.join(root, 'bench.py')] + extra, stdout=subprocess.PIPE, stderr=subprocess.PIPE,
+                             text=True, env=env, timeout=600)
+        assert res.returncode == 2 and not res.stdout.strip(), (extra, res.stderr[-500:])
+    assert not os.path.exists(tmp_path / 'out')
+
+
 def test_installed_reference_agrees_with_the_oracle_on_the_headline_model():
     """`baseline/_ref` (the unmodified reference, pip-installed by `__graft_entry__.build()`; absent on boxes without
     /root/reference and then skipped): the ln_prob composition that `bench.py --impl reference` times equals the oracle's
