@@ -66,14 +66,26 @@ static __device__ long long gf_stage_last;
  * subnormal range.  Eigenvectors are invariant under the scaling. */
 #define GFP_MASS_SCALE 1180591620717411303424.0 /* 2^70 */
 
-/* Relative eigenvalue gap (in units of 2 sqrt(Q)) below which the closed-form path hands over
- * to Jacobi: the closed form loses accuracy like eps/gap^2, Jacobi like eps/gap. */
-#ifdef GFP_FAST_MIN_SIN2
-#define GFP_FAST_MIN_SIN2_OVERRIDDEN 1 /* developer builds with another threshold use the fp64 compare */
-#else
-#define GFP_FAST_MIN_SIN2 1.4e-6 /* sin^2(phi/3): gap = sqrt(3 * sin^2) ~ 2.0e-3 */
+/* sin^2(phi/3) below which the closed-form path hands the bin over to the deflation refinement: the closed form loses
+ * accuracy like eps/relgap^2, the refinement like eps/relgap (relgap = closest pair's splitting / spectral spread =
+ * (2/sqrt(3)) sin(phi/3) for a close pair).  4.7e-6 is relgap 2.5e-3, where the closed form's worst |V|^2 error over
+ * 1e6 Haar-random spectra is 3.8e-11; at the former 1.4e-6 (relgap 1.37e-3) it was 1.29e-10, above the 1e-10
+ * tolerance on fr (tests/test_eigen_conditioning.py::test_harness_closed_form_error_at_the_fast_path_cut). */
+#ifndef GFP_FAST_MIN_SIN2
+#define GFP_FAST_MIN_SIN2 4.7e-6
 #endif
 #define GFP_ILL_GAP 1e-6
+
+/* High 32-bit word of a positive, normal double at compile time (exact: scaling by two and the mantissa's top 20 bits
+ * are exact operations).  The device compares sin^2(phi/3) with the threshold on this word. */
+constexpr unsigned gfp_hiword_pos(double x) {
+    int e = 0;
+    while (x >= 2.0) { x *= 0.5; ++e; }
+    while (x < 1.0) { x *= 2.0; --e; }
+    return ((unsigned)(e + 1023) << 20) | (unsigned)((x - 1.0) * 1048576.0);
+}
+constexpr unsigned GFP_FAST_MIN_SIN2_HI = gfp_hiword_pos(GFP_FAST_MIN_SIN2);
+static_assert(GFP_FAST_MIN_SIN2_HI > 0x00100000u && GFP_FAST_MIN_SIN2_HI < 0x7FF00000u, "the fast-path threshold must be positive and finite");
 
 /* ------------------------------------------------------------------ fast fp64 helpers */
 
@@ -348,10 +360,11 @@ GF_HD bool gfp_eig_core(double e0, double e1, double k0, double k1, double Q, do
     out.x11 = n11 * i1;
     /* Q > tiny also rejects NaN; s2 >= limit rejects close pairs, NaN and negative round-off.  On the device
      * both tests read the exponent fields with integer instructions (unsigned range checks: positive, finite,
-     * above the threshold's high word) instead of two compares on the fp64 pipe. */
-#if defined(__CUDA_ARCH__) && !defined(GFP_FAST_MIN_SIN2_OVERRIDDEN)
+     * above the threshold's high word) instead of two compares on the fp64 pipe.  The high word ignores the low 32 bits
+     * of the threshold: the device's cut sits at most 2^-20 relative below the host's. */
+#if defined(__CUDA_ARCH__)
     const unsigned hq = (unsigned)__double2hiint(Q), hs = (unsigned)__double2hiint(s2);
-    return (hq - 0x05E00000u < 0x7FF00000u - 0x05E00000u) && (hs - 0x3EB77CF4u < 0x7FF00000u - 0x3EB77CF4u); /* Q > ~1e-280, s2 >= 1.4e-6 */
+    return (hq - 0x05E00000u < 0x7FF00000u - 0x05E00000u) && (hs - GFP_FAST_MIN_SIN2_HI < 0x7FF00000u - GFP_FAST_MIN_SIN2_HI); /* Q > ~1e-280, s2 >= GFP_FAST_MIN_SIN2 */
 #else
     return (Q > 1e-280) && (s2 >= GFP_FAST_MIN_SIN2);
 #endif
@@ -483,17 +496,20 @@ GF_HD bool gfp_pencil_x4_fast(const gfp_pencil_P& p, const gfp_pencil_T& t, doub
  */
 GF_HD_NOINLINE double gfp_herm3_jacobi(const gfp_herm3& h, double* lam, double* vr, double* vi) {
     double hr[9], hi[9];
-    /* scale to unit max-norm (exact power-of-two free scaling is not needed: eigenvectors are
-     * scale invariant, eigenvalues are rescaled at the end) */
+    /* scale the largest entry into [1, 2) by an EXACT power of two 2^-ex taken from its exponent (subnormals included):
+     * the squares of the rotations can then neither overflow nor underflow at any input scale, the eigenvectors are
+     * the same bits at every power-of-two scale, and the eigenvalues are rescaled exactly.  A reciprocal of the
+     * largest entry would overflow for a subnormal one and round the entries.  Non-finite input is not scaled
+     * (ex = 0) and comes out non-finite. */
     double mx = fmax(fmax(fabs(h.d0), fabs(h.d1)), fabs(h.d2));
     mx = fmax(mx, fmax(fmax(fabs(h.ar), fabs(h.ai)), fmax(fmax(fabs(h.br), fabs(h.bi)), fmax(fabs(h.cr), fabs(h.ci)))));
-    const double sc = (mx > 0.0 && mx < 1e300) ? 1.0 / mx : 1.0;
-    hr[0] = h.d0 * sc; hi[0] = 0.0;
-    hr[4] = h.d1 * sc; hi[4] = 0.0;
-    hr[8] = h.d2 * sc; hi[8] = 0.0;
-    hr[1] = h.ar * sc; hi[1] = h.ai * sc; hr[3] = hr[1]; hi[3] = -hi[1];
-    hr[2] = h.br * sc; hi[2] = h.bi * sc; hr[6] = hr[2]; hi[6] = -hi[2];
-    hr[5] = h.cr * sc; hi[5] = h.ci * sc; hr[7] = hr[5]; hi[7] = -hi[5];
+    const int ex = (mx > 0.0 && mx <= 1.7976931348623157e308) ? ilogb(mx) : 0;
+    hr[0] = scalbn(h.d0, -ex); hi[0] = 0.0;
+    hr[4] = scalbn(h.d1, -ex); hi[4] = 0.0;
+    hr[8] = scalbn(h.d2, -ex); hi[8] = 0.0;
+    hr[1] = scalbn(h.ar, -ex); hi[1] = scalbn(h.ai, -ex); hr[3] = hr[1]; hi[3] = -hi[1];
+    hr[2] = scalbn(h.br, -ex); hi[2] = scalbn(h.bi, -ex); hr[6] = hr[2]; hi[6] = -hi[2];
+    hr[5] = scalbn(h.cr, -ex); hi[5] = scalbn(h.ci, -ex); hr[7] = hr[5]; hi[7] = -hi[5];
     for (int k = 0; k < 9; ++k) { vr[k] = (k % 4 == 0) ? 1.0 : 0.0; vi[k] = 0.0; }
 
     for (int sweep = 0; sweep < 24; ++sweep) {
@@ -538,7 +554,7 @@ GF_HD_NOINLINE double gfp_herm3_jacobi(const gfp_herm3& h, double* lam, double* 
         }
     }
     const double l0 = hr[0], l1 = hr[4], l2 = hr[8];
-    lam[0] = l0 * mx; lam[1] = l1 * mx; lam[2] = l2 * mx;
+    lam[0] = scalbn(l0, ex); lam[1] = scalbn(l1, ex); lam[2] = scalbn(l2, ex);
     const double g01 = fabs(l0 - l1), g02 = fabs(l0 - l2), g12 = fabs(l1 - l2);
     const double spread = fmax(g01, fmax(g02, g12));
     const double gmin = fmin(g01, fmin(g02, g12));

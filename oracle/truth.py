@@ -61,10 +61,7 @@ def _mp_u(ang, mp):
         [s23 * s12 - c23 * s13 * ep * c12, -s23 * c12 - c23 * s13 * ep * s12, c23 * c13]])
 
 
-def mp_bsm_fr_bin(sm_angles, mass, np_angles, loglam, dim, energy, source, dps=50):
-    """u_to_fr(source, eigvecs(H)) for one energy, all in mpmath."""
-    import mpmath as mp
-    mp.mp.dps = dps
+def _mp_bin_hamiltonian(sm_angles, mass, np_angles, loglam, dim, energy, mp):
     u = _mp_u(sm_angles, mp)
     n = _mp_u(np_angles, mp)
     m = mp.diag([0, mp.mpf(float(mass[0])), mp.mpf(float(mass[1]))])
@@ -72,8 +69,14 @@ def mp_bsm_fr_bin(sm_angles, mass, np_angles, loglam, dim, energy, source, dps=5
     s = mp.diag([0, sc2 / 100, sc2])
     e = mp.mpf(float(energy))
     h = (u * m * u.H) / (2 * e) + (e ** (dim - 3)) * (n * s * n.H)
-    h = (h + h.H) / 2
-    _, v = mp.eighe(h)
+    return (h + h.H) / 2
+
+
+def mp_bsm_fr_bin(sm_angles, mass, np_angles, loglam, dim, energy, source, dps=50):
+    """u_to_fr(source, eigvecs(H)) for one energy, all in mpmath."""
+    import mpmath as mp
+    mp.mp.dps = dps
+    _, v = mp.eighe(_mp_bin_hamiltonian(sm_angles, mass, np_angles, loglam, dim, energy, mp))
     p = [[abs(v[a, i]) ** 2 for i in range(3)] for a in range(3)]
     src = [mp.mpf(float(x)) for x in source]
     tot = sum(src)
@@ -100,3 +103,16 @@ def mp_flux_averaged_fr(sm_angles, mass, np_angles, loglam, dim, binning, source
         acc = [a + mp.mpf(float(w)) * x for a, x in zip(acc, f)]
     tot = sum(acc)
     return np.array([float(a / tot) for a in acc])
+
+
+def mp_bin_relgaps(sm_angles, mass, np_angles, loglam, dim, binning, dps=50):
+    """Relative gap of every energy bin's Hamiltonian in mpmath: the closest eigenvalue pair's splitting divided by
+    the spectral spread (the quantity the kernels' ILL_COND flag and fast-path cut refer to)."""
+    import mpmath as mp
+    mp.mp.dps = dps
+    binning = np.asarray(binning, dtype=np.float64)
+    out = []
+    for ec in np.sqrt(binning[:-1] * binning[1:]):
+        lam = sorted(mp.eighe(_mp_bin_hamiltonian(sm_angles, mass, np_angles, loglam, dim, ec, mp), eigvals_only=True))
+        out.append(float(min(lam[1] - lam[0], lam[2] - lam[1]) / (lam[2] - lam[0])))
+    return np.array(out)

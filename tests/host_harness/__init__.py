@@ -147,3 +147,12 @@ def ndtri(p):
     z, ok = np.empty_like(p), np.empty(p.shape[0], dtype=np.uint8)
     load().hh_ndtri(_p(p), C.c_int64(p.shape[0]), _p(z), _p(ok))
     return z, ok.astype(bool)
+
+
+def fast_min_sin2():
+    """(GFP_FAST_MIN_SIN2, the high word the device compares sin^2(phi/3) with)."""
+    thr = C.c_double()
+    fn = load().hh_fast_min_sin2
+    fn.restype = C.c_uint
+    hi = fn(C.byref(thr))
+    return thr.value, hi

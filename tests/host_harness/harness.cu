@@ -207,3 +207,9 @@ extern "C" int hh_lnprob_rebuild(const gf_model* model, const double* theta, int
     }
     return 0;
 }
+
+/* the fast path's sin^2(phi/3) threshold and the high word the device compares with */
+extern "C" unsigned hh_fast_min_sin2(double* thr) {
+    *thr = GFP_FAST_MIN_SIN2;
+    return GFP_FAST_MIN_SIN2_HI;
+}
