@@ -73,6 +73,11 @@ class EnsembleConfig(C.Structure):
                 ('step0', C.c_int64), ('thin', C.c_int64), ('a', C.c_double), ('seed', C.c_uint64), ('chain0', C.c_int64), ('mode', C.c_int32), ('cluster_blocks', C.c_int32)]
 
 
+class ProfileConfig(C.Structure):
+    _fields_ = [('seed', C.c_uint64), ('task0', C.c_int64), ('nstarts', C.c_int32), ('max_evals', C.c_int32),
+                ('ftol', C.c_double), ('xtol', C.c_double)]
+
+
 _P = C.c_void_p
 _SIGNATURES = {
     'gf_abi_version': (C.c_int, []),
@@ -101,6 +106,7 @@ _SIGNATURES = {
     'gf_scan_evidence': (C.c_int, [C.POINTER(Model), C.POINTER(ScanConfig), _P, _P]),
     'gf_scan_evidence_grid_workspace': (C.c_uint64, [C.c_int32]),
     'gf_scan_evidence_grid': (C.c_int, [C.POINTER(Model), C.POINTER(ScanConfig), _P, C.c_int32, _P, _P, C.c_uint64, _P]),
+    'gf_profile_grid': (C.c_int, [C.POINTER(Model), C.POINTER(ProfileConfig), _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
     'gf_coverage_mask': (C.c_int, [_P, C.c_int64, C.c_double, _P, C.POINTER(C.c_uint64), _P]),
     'gf_hist_smooth': (C.c_int, [_P, C.c_int32, C.c_uint64, _P, C.c_int32, _P, _P, _P]),
     'gf_coverage_mask_f64': (C.c_int, [_P, C.c_int64, C.c_double, _P, C.POINTER(C.c_double), C.POINTER(C.c_uint64), _P]),
@@ -129,7 +135,7 @@ def load():
             fn.restype, fn.argtypes = res, args
         if lib.gf_abi_version() != 1:
             raise GolemFlavorError('golemflavor_b200: ABI version mismatch, rebuild the library')
-        for which, struct in enumerate((Model, ScanConfig, PriorDim, EnsembleConfig)):
+        for which, struct in enumerate((Model, ScanConfig, PriorDim, EnsembleConfig, ProfileConfig)):
             if lib.gf_sizeof(which) != C.sizeof(struct):
                 raise GolemFlavorError('golemflavor_b200: layout of {0} differs between _lib.py ({1} B) and the '
                                        'library ({2} B)'.format(struct.__name__, C.sizeof(struct), lib.gf_sizeof(which)))

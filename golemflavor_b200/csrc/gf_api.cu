@@ -42,7 +42,8 @@ extern "C" int gf_abi_version(void) { return GF_ABI_VERSION; }
 extern "C" const char* gf_last_error(void) { return g_last_error; }
 extern "C" uint64_t gf_launch_count(void) { return g_gf_launches.load(); }
 extern "C" uint64_t gf_sizeof(int32_t which) {
-    return which == 0 ? sizeof(gf_model) : which == 1 ? sizeof(gf_scan_config) : which == 2 ? sizeof(gf_prior_dim) : which == 3 ? sizeof(gf_ensemble_config) : 0;
+    return which == 0 ? sizeof(gf_model) : which == 1 ? sizeof(gf_scan_config) : which == 2 ? sizeof(gf_prior_dim) : which == 3 ? sizeof(gf_ensemble_config)
+         : which == 4 ? sizeof(gf_profile_config) : 0;
 }
 
 extern "C" int gf_device_info(int32_t* sm_count, int32_t* cc_major, int32_t* cc_minor, int32_t* clock_khz) {

@@ -21,7 +21,7 @@ from .enums import ParamTag, PriorsCateg, Texture, enum_name
 from .param import Param, ParamSet
 
 __all__ = ['sm_paramset', 'scan_paramset', 'scan_model', 'scan_histogram', 'scan_samples', 'ternary_histogram',
-           'shard_range', 'allreduce_counts', 'coverage_mask', 'scan_evidence', 'scan_evidence_grid']
+           'shard_range', 'allreduce_counts', 'coverage_mask', 'scan_evidence', 'scan_evidence_grid', 'scan_profile_grid']
 
 DEFAULT_BINNING = np.logspace(np.log10(6e4), np.log10(1e7), 21)  # fr.py:283-285
 
@@ -275,3 +275,42 @@ def scan_evidence_grid(fm, scales, count, seed=26, first_index=0, distributed=Tr
     h = lse.cpu().numpy()
     with np.errstate(divide='ignore'):
         return np.where(h[:, 1] > 0, h[:, 0] + np.log(h[:, 1]) - np.log(count), -np.inf)
+
+
+# defaults of the profile optimiser, from the host-harness study recorded in DESIGN.md (K3c)
+PROFILE_NSTARTS = 64
+PROFILE_MAX_EVALS = 6000
+PROFILE_FTOL = 1e-10
+PROFILE_XTOL = 1e-7
+
+
+def scan_profile_grid(fm, scales, nstarts=PROFILE_NSTARTS, seed=27, task0=0, max_evals=PROFILE_MAX_EVALS, ftol=PROFILE_FTOL,
+                      xtol=PROFILE_XTOL):
+    """Profile likelihood at every frozen scale of ``scales`` (log10 Lambda) in ONE launch (``gf_profile_grid``): the maximum of
+    ``ln_prob`` over the model's columns inside their prior box, by bounded Nelder-Mead from ``nstarts`` starts per scale (the
+    prior means, then prior draws).  The model must not sample the scale (``args.fixed_scale``).  ``task0`` is the global index
+    of ``scales[0]``: a scale's result depends on ``(seed, task0 + s, nstarts)`` only, however the scales are split over calls.
+    Returns a dict of NumPy arrays: ``best`` [ns], ``argmax`` [ns, ndim], ``fr`` [ns, 3] (composition at the argmax),
+    ``status`` [ns] (its GF_ST_* bits), ``nevals`` [ns] (objective evaluations over all starts), ``nconverged`` [ns]
+    (starts that converged before ``max_evals``)."""
+    torch = _lib.torch_cuda()
+    best, argmax, fr, st, counts = _profile_launch(torch, fm, scales, nstarts, seed, task0, max_evals, ftol, xtol)
+    c = counts.cpu().numpy()
+    return dict(best=best.cpu().numpy(), argmax=argmax.cpu().numpy(), fr=fr.cpu().numpy(), status=st.cpu().numpy(), nevals=c[:, 0],
+                nconverged=c[:, 1])
+
+
+def _profile_launch(torch, fm, scales, nstarts, seed, task0, max_evals=PROFILE_MAX_EVALS, ftol=PROFILE_FTOL, xtol=PROFILE_XTOL):
+    """Enqueue ``gf_profile_grid`` on torch's current stream: (best, argmax, fr, status, counts) as CUDA tensors."""
+    sc = torch.as_tensor(np.ascontiguousarray(scales, dtype=np.float64).ravel()).cuda()
+    ns = int(sc.numel())
+    best = torch.empty((ns,), dtype=torch.float64, device='cuda')
+    argmax = torch.empty((ns, fm.ndim), dtype=torch.float64, device='cuda')
+    fr = torch.empty((ns, 3), dtype=torch.float64, device='cuda')
+    st = torch.empty((ns,), dtype=torch.uint8, device='cuda')
+    counts = torch.empty((ns, 2), dtype=torch.int64, device='cuda')
+    cfg = _lib.ProfileConfig(seed=int(seed), task0=int(task0), nstarts=int(nstarts), max_evals=int(max_evals), ftol=float(ftol),
+                             xtol=float(xtol))
+    _lib.check(_lib.load().gf_profile_grid(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, _lib.ptr(best), _lib.ptr(argmax), _lib.ptr(fr),
+                                           _lib.ptr(st), _lib.ptr(counts), _lib.stream_ptr(torch)))
+    return best, argmax, fr, st, counts

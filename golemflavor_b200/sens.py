@@ -19,9 +19,9 @@ from . import model as _model
 from .enums import ParamTag, Texture
 from .mcmc import DeviceEnsembleSampler
 from .param import Param, ParamSet
-from .scan import DEFAULT_BINNING, _dist, shard_range, sm_paramset
+from .scan import DEFAULT_BINNING, PROFILE_NSTARTS, _dist, _profile_launch, shard_range, sm_paramset
 
-__all__ = ['scale_grid', 'sweep_paramset', 'sweep', 'evidence_grid', 'get_limit', 'limits', 'BAYES_K']
+__all__ = ['scale_grid', 'sweep_paramset', 'sweep', 'evidence_grid', 'profile_grid', 'get_limit', 'limits', 'BAYES_K', 'FREQ_CL']
 
 
 def scale_grid(dimension, segments):
@@ -184,6 +184,65 @@ def evidence_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.O
     return ev
 
 
+def _grid_model(dim, texture, src, inj, smearing, binning):
+    """The six SM nuisance parameters with the scale frozen (``sens.py:261-266``), built exactly as ``evidence_grid`` builds
+    its model; the kernel substitutes each grid scale."""
+    args = Namespace(source_ratio=src / src.sum(), dimension=int(dim), texture=texture, binning=np.asarray(binning),
+                     no_bsm=False, injected_ratio=inj / inj.sum(), smearing=float(smearing), fixed_scale=-100.0)
+    return _model.flatten(args, None, ParamSet(sm_paramset(with_mass=True)))
+
+
+def profile_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, source_ratio=(1, 2, 0),
+                 injected_ratio=(1, 1, 1), smearing=0.02, nstarts=PROFILE_NSTARTS, seed=27, binning=DEFAULT_BINNING,
+                 distributed=True, return_argmax=False):
+    """Profile likelihood per (dimension, scale) grid point: the frequentist statistic of ``scripts/sens.py``
+    (``StatCateg.FREQUENTIST``, which the reference takes from GolemFit's profiled fit, ``gf.get_llh_freq``).  With the Gaussian
+    flavor-ratio likelihood it is the maximum of ``ln_prob`` over the six SM nuisance parameters inside their prior box, the
+    scale frozen at the grid value; the Gaussian priors act as penalty terms.  Returns ``{dimension: array[segments, 2]}`` of
+    (scale, profile ln_prob), the layout of ``evidence_grid``; ``get_limit(..., args=Namespace(stat_method=FREQUENTIST))``
+    turns it into a limit.  With ``return_argmax`` also ``{dimension: array[segments, 6]}`` of the maximising parameters.
+
+    ONE launch per dimension (``gf_profile_grid``: one block per scale, one thread per start), on one stream per dimension.
+    The grid points are sharded over the ranks of the process group (``task0`` = index of the scale in its dimension's grid)
+    and the disjoint rows are merged with one all-reduce: the result is the same for any number of ranks."""
+    torch = _lib.torch_cuda()
+    dist = _dist() if distributed else None
+    rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
+    src = np.asarray(source_ratio, dtype=np.float64)
+    inj = np.asarray(injected_ratio, dtype=np.float64)
+    dims = [int(d) for d in dimensions]
+    segments = int(segments)
+    grid = [(k, s) for k in range(len(dims)) for s in range(segments)]
+    start, count = shard_range(len(grid), rank, world)
+    ndim = len(sm_paramset(with_mass=True))
+    rows = np.zeros((len(grid), 1 + ndim))
+    cur = torch.cuda.current_stream()
+    pending = []
+    for k, dim in enumerate(dims):
+        mine = [s for kk, s in grid[start:start + count] if kk == k]
+        if not mine:
+            continue
+        fm = _grid_model(dim, texture, src, inj, smearing, binning)
+        scales = scale_grid(dim, segments)[mine[0]:mine[-1] + 1]
+        stream = _dim_stream(torch, dim)
+        stream.wait_stream(cur)
+        with torch.cuda.stream(stream):
+            out = _profile_launch(torch, fm, scales, nstarts, seed, mine[0])
+        pending.append((stream, k * segments + mine[0], out))
+    for stream, row0, (best, argmax, _, _, _) in pending:
+        stream.synchronize()
+        rows[row0:row0 + best.numel(), 0] = best.cpu().numpy()
+        rows[row0:row0 + best.numel(), 1:] = argmax.cpu().numpy()
+    if dist and world > 1:
+        t = torch.as_tensor(rows).cuda()
+        dist.all_reduce(t, op=dist.ReduceOp.SUM)                   # disjoint rows: sum == gather
+        rows = t.cpu().numpy()
+    prof = {d: np.column_stack([scale_grid(d, segments), rows[k * segments:(k + 1) * segments, 0]]) for k, d in enumerate(dims)}
+    if return_argmax:
+        return prof, {d: rows[k * segments:(k + 1) * segments, 1:].copy() for k, d in enumerate(dims)}
+    return prof
+
+
 _WORK = {}
 
 
@@ -197,9 +256,10 @@ def _workspace(torch, nbytes):
 
 
 BAYES_K = 1.   # golemflavor/plot.py:82: "Strong degree of belief"
+FREQ_CL = 0.90  # confidence level of the frequentist limit
 
 
-def get_limit(scales, statistic, args=None, mask_initial=False, return_interp=False, bayes_k=BAYES_K, verbose=False):
+def get_limit(scales, statistic, args=None, mask_initial=False, return_interp=False, bayes_k=BAYES_K, verbose=False, cl=FREQ_CL):
     """Limit on the new-physics scale from the evidence curve of one operator dimension (``plot.get_limit``,
     ``plot.py:149-213``; the consumer of the ``(scale, lnZ)`` pairs ``scripts/sens.py:289-294`` stores).
 
@@ -209,14 +269,24 @@ def get_limit(scales, statistic, args=None, mask_initial=False, return_interp=Fa
     (conversion to the standard SME coefficient, ``plot.py:208-210``).  Same outcomes as the reference: ``AssertionError``
     ('Discovered LV!') if the null point itself is disfavoured by more than the threshold, ``None`` when no splined point
     crosses it, when the contour is peaked (>= 2 grid points beyond the crossing fall 0.1 below the threshold) or when
-    fewer than 2 grid points beyond the crossing reach it; ``return_interp`` returns ``(splined scales, reduced evidence)``."""
+    fewer than 2 grid points beyond the crossing reach it; ``return_interp`` returns ``(splined scales, reduced evidence)``.
+
+    With ``args.stat_method == StatCateg.FREQUENTIST`` ``statistic`` is the profile ln_prob (``profile_grid``) and only the
+    threshold changes: ``chi2.ppf(cl, 1) / 2`` in ln L, i.e. Wilks' -2 Delta ln L > chi^2 with one degree of freedom; the
+    spline and every rule above are the same.  No fixture pins this branch against the reference: its frequentist value
+    comes from GolemFit (``gf.get_llh_freq``).  The rule is this project's definition, and Wilks' theorem is an
+    approximation where the scale sits at a bounded end of its range."""
     from scipy.interpolate import splev, splprep
     scales = np.asarray(scales, dtype=np.float64)
     statistic = np.asarray(statistic, dtype=np.float64)
     thr = np.log(10 ** bayes_k)
-    if args is not None and getattr(args, 'stat_method', None) is not None and \
-            str(getattr(args.stat_method, 'name', args.stat_method)).upper() != 'BAYESIAN':
-        raise NotImplementedError
+    if args is not None and getattr(args, 'stat_method', None) is not None:
+        method = str(getattr(args.stat_method, 'name', args.stat_method)).upper()
+        if method == 'FREQUENTIST':
+            from scipy.stats import chi2
+            thr = chi2.ppf(cl, 1) / 2.
+        elif method != 'BAYESIAN':
+            raise NotImplementedError
     if (statistic[0] - np.max(statistic)) > thr:
         raise AssertionError('Discovered LV!')
     tck, _ = splprep([scales, statistic], s=0)

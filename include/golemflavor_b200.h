@@ -125,7 +125,7 @@ typedef struct gf_scan_config {
 
 /* ---- library ---------------------------------------------------------- */
 int gf_abi_version(void);
-/* sizeof(gf_model) / gf_scan_config / gf_prior_dim / gf_ensemble_config for which = 0 / 1 / 2 / 3: lets a
+/* sizeof(gf_model) / gf_scan_config / gf_prior_dim / gf_ensemble_config / gf_profile_config for which = 0 / 1 / 2 / 3 / 4: lets a
  * foreign-language binding verify its struct layout at load time. */
 uint64_t gf_sizeof(int32_t which);
 const char* gf_last_error(void);
@@ -212,6 +212,34 @@ int gf_scan_evidence(const gf_model* model, const gf_scan_config* cfg, double* d
 uint64_t gf_scan_evidence_grid_workspace(int32_t nscales);
 int gf_scan_evidence_grid(const gf_model* model, const gf_scan_config* cfg, const double* d_scales /*[nscales]*/, int32_t nscales,
                           double* d_lse /*[nscales][2]*/, void* d_work, uint64_t work_bytes, void* stream);
+/*
+ * Profile likelihood on the same grid: the frequentist statistic of scripts/sens.py (StatCateg.FREQUENTIST, whose value the
+ * reference takes from GolemFit's profiled fit, gf.get_llh_freq / Likelihood.GF_FREQ).  For each frozen scale
+ * d_scales[s] = log10(Lambda_s) of a model that does not sample the scale (col_scale = -1), d_best[s] = the maximum of ln_prob
+ * (llh.ln_prob: prior terms included) over every model column inside its prior box.  Task (s, k) is bounded Nelder-Mead
+ * (Gao & Han's adaptive coefficients) in coordinates scaled per column (sigma of a Gaussian prior, a tenth of a uniform box)
+ * from start k: start 0 = the prior means clipped to the box (the centre of a uniform box), start k >= 1 = the prior draw of
+ * the scans with sample index (task0 + s) * nstarts + k (see gf_scan_config).  It converges when the spread of ln_prob over
+ * the simplex is <= ftol and its extent <= xtol in every scaled coordinate, restarts from the best vertex with a fresh
+ * simplex, and stops when a restart gains < ftol or after max_evals evaluations.  The best start wins (ties: the lower k),
+ * so a scale's result depends on (seed, task0 + s, nstarts) only: not on how the scales are split over calls or GPUs.
+ * Optional outputs: d_argmax[s] = the maximising theta, d_fr[s] = its measured composition, d_status[s] = its status bits
+ * (| GF_ST_NON_FINITE if any evaluation of the scale was not finite; such values count as -inf), d_counts[s] =
+ * {evaluations over all starts, starts that converged before max_evals}.  One launch: one block per scale, one thread per
+ * start; the simplices take (ndim + 1)^2 * nstarts * 8 bytes of shared memory per block (GF_ERR_ARG beyond the device's limit).
+ */
+typedef struct gf_profile_config {
+    uint64_t seed;      /* Philox key of the starts                                   */
+    int64_t task0;      /* global index of d_scales[0]: shard / split offset          */
+    int32_t nstarts;    /* starts per scale, multiple of 32, <= 256                   */
+    int32_t max_evals;  /* objective evaluations per start                            */
+    double ftol;        /* spread of ln_prob over the simplex                         */
+    double xtol;        /* simplex diameter in scaled coordinates                     */
+} gf_profile_config;
+int gf_profile_grid(const gf_model* model, const gf_profile_config* cfg, const double* d_scales, int32_t nscales,
+                    double* d_best /*[nscales]*/, double* d_argmax /*[nscales][ndim] or NULL*/,
+                    double* d_fr /*[nscales][3] or NULL*/, uint8_t* d_status /*[nscales] or NULL*/,
+                    int64_t* d_counts /*[nscales][2] or NULL: evaluations, starts that converged*/, void* stream);
 /* Highest-density coverage region of a histogram (plot.flavor_contour, plot.py:372-384: normalise,
  * sort cells by content, cumulative sum, `thres = searchsorted(cumsum, coverage/100)`, mask the first
  * `thres` cells).  d_mask[i] = 1 for the cells inside the region.  h_info (host, optional) receives
