@@ -482,6 +482,108 @@ GF_HD void gf_point_fr_scales(const gf_dev_model& m, const gf_point& q, int ns, 
     }
 }
 
+/*
+ * The energy-bin loop of gf_bin_loop (same fast path, same rare refinement, ILP interleaved chains, LANES = 1) with a
+ * source-independent result: the bin-width-weighted sums of the transition P = X X^T in its three independent entries,
+ * A[0..2] = sum_b w_b (P00, P01, P11) (gfp_x4_transition).  gfp_transition_fr turns them into the composition of any
+ * source.  Returns the status bits of the eigen stage.
+ */
+template <int ILP, class TPART, class MATS>
+GF_HD unsigned gf_bin_loop_transition(const gf_dev_model& m, const gfp_pencil_P& pp, const TPART& pt, const MATS& mats, double lam, double* A) {
+    unsigned st = 0u;
+    double a00 = 0.0, a01 = 0.0, a11 = 0.0;
+    int b = 0;
+    if (ILP > 1) {
+        for (; b + ILP - 1 < m.nbins; b += ILP) {
+            gfp_x4 x[ILP];
+            bool ok = true;
+#pragma unroll
+            for (int i = 0; i < ILP; ++i) ok = gfp_pencil_x4_fast(pp, pt, lam * m.g[b + i], x[i]) && ok;
+            if (!ok) {
+#pragma unroll
+                for (int i = 0; i < ILP; ++i) {
+                    gfp_x4 again;
+                    if (!gfp_pencil_x4_fast(pp, pt, lam * m.g[b + i], again)) {
+                        gfp_x4 slow;
+                        st |= gf_refine_bin(mats, lam * m.g[b + i], &slow);
+                        x[i] = slow;
+                    }
+                }
+            }
+#pragma unroll
+            for (int i = 0; i < ILP; ++i) {
+                double p00, p01, p11;
+                gfp_x4_transition(x[i], p00, p01, p11);
+                const double wd = m.width[b + i];
+                a00 = fma(wd, p00, a00);
+                a01 = fma(wd, p01, a01);
+                a11 = fma(wd, p11, a11);
+            }
+        }
+    }
+    for (; b < m.nbins; ++b) {
+        const double rho = lam * m.g[b];
+        gfp_x4 x;
+        if (!gfp_pencil_x4_fast(pp, pt, rho, x)) {
+            gfp_x4 slow;
+            st |= gf_refine_bin(mats, rho, &slow);
+            x = slow;
+        }
+        double p00, p01, p11;
+        gfp_x4_transition(x, p00, p01, p11);
+        const double wd = m.width[b];
+        a00 = fma(wd, p00, a00);
+        a01 = fma(wd, p01, a01);
+        a11 = fma(wd, p11, a11);
+    }
+    A[0] = a00;
+    A[1] = a01;
+    A[2] = a11;
+    return st;
+}
+
+/*
+ * The twin of gf_point_fr_scales for many sources at once: the same once-per-point set-up (PMNS, H0, T, pencil, refinement
+ * matrices), then `emit(s, A, status)` per scale with the transition sums A of gf_bin_loop_transition at lam_of(s).  The
+ * model's source (fixed_src, sampled source columns) is not used.  status carries the eigen-stage bits and
+ * GFP_ST_NON_FINITE; unitarity is a property of a composition, hence of a source, and is not tested here.
+ */
+template <int SPEC, int ILP, class LamOf, class Emit, class ThetaSrc = gf_no_src>
+GF_HD void gf_point_transition_scales(const gf_dev_model& m, const gf_point& q, int ns, LamOf lam_of, Emit emit, const ThetaSrc& src = ThetaSrc()) {
+    static_assert(!GF_SPEC_IS_SM(SPEC), "the scale grid needs the BSM path");
+    gfp_herm3 h0, T;
+    double m1, m2;
+    gf_point_matrices<SPEC>(m, q, h0, T, m1, m2);
+    auto finish = [&](int s, unsigned st, double* A) {
+        if (!(fabs(A[0]) + fabs(A[1]) + fabs(A[2]) < 1e300)) st |= GFP_ST_NON_FINITE;
+        emit(s, A, st);
+    };
+    auto run = [&](const auto& mats) {
+        if (GF_SPEC_IS_FIXED(SPEC)) {
+            const gfp_pencil_P pp = gfp_make_pencil_P(h0, m1, m2, m.T, m.penT.te, m.adjT);
+            for (int s = 0; s < ns; ++s) {
+                double A[3];
+                const unsigned st = gf_bin_loop_transition<ILP>(m, pp, m.penT, mats, lam_of(s), A);
+                finish(s, st, A);
+            }
+        } else {
+            const bool npf = GF_SPEC_IS_NPFREE(SPEC) || m.np_free;
+            const gfp_pencil_T pt = gfp_make_pencil_T(T);
+            const gfp_pencil_P pp = gfp_make_pencil_P(h0, m1, m2, T, pt.te, npf ? gfp_adj_tf(pt.te, T) : m.adjT);
+            for (int s = 0; s < ns; ++s) {
+                double A[3];
+                const unsigned st = gf_bin_loop_transition<ILP>(m, pp, pt, mats, lam_of(s), A);
+                finish(s, st, A);
+            }
+        }
+    };
+    if constexpr (std::is_same<ThetaSrc, gf_no_src>::value) {
+        run(gf_mats_ptr{&h0, GF_SPEC_IS_FIXED(SPEC) ? &m.T : &T});
+    } else {
+        run(gf_mats_rebuild<SPEC, ThetaSrc>{&m, src});
+    }
+}
+
 GF_HD int gf_model_gauss_mask(const gf_dev_model& m) {
     int mask = 0;
     for (int k = 0; k < m.ndim; ++k) mask |= (m.kind[k] != GF_PRIOR_UNIFORM) << k;

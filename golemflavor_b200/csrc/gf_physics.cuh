@@ -795,6 +795,39 @@ GF_HD void gfp_mix4(const gfp_x4& x, double s2, double sd0, double sd1, double S
     f1 = fma(x.x10, u0, fma(x.x11, u1, w2));
 }
 
+/* The flavor transition P = X X^T of a doubly stochastic X is symmetric and doubly stochastic, so three numbers determine
+ * it: P00 = sum_i X_0i^2, P01 = sum_i X_0i X_1i, P11 = sum_i X_1i^2 (the third row and column follow from the unit sums).
+ * From the four independent entries of gfp_x4; X_a2 = 1 - X_a0 - X_a1. */
+GF_HD void gfp_x4_transition(const gfp_x4& x, double& p00, double& p01, double& p11) {
+    const double x02 = 1.0 - x.x00 - x.x01, x12 = 1.0 - x.x10 - x.x11;
+    p00 = fma(x.x00, x.x00, fma(x.x01, x.x01, x02 * x02));
+    p01 = fma(x.x00, x.x10, fma(x.x01, x.x11, x02 * x12));
+    p11 = fma(x.x10, x.x10, fma(x.x11, x.x11, x12 * x12));
+}
+
+/* A source composition s in the form gfp_transition_fr consumes, for bin-width sums W = sum_b w_b:
+ * sd0 = s0 - s2, sd1 = s1 - s2, ws2 = W s2, inv_sw = 1 / (S W) with S = s0 + s1 + s2. */
+struct gfp_src_consts {
+    double sd0, sd1, ws2, inv_sw;
+};
+GF_HD gfp_src_consts gfp_source_consts(double s0, double s1, double s2, double W) {
+    gfp_src_consts c;
+    c.sd0 = s0 - s2;
+    c.sd1 = s1 - s2;
+    c.ws2 = W * s2;
+    c.inv_sw = 1.0 / ((s0 + s1 + s2) * W);
+    return c;
+}
+
+/* flux_averaged_BSMu (fr.py:441-457) of ANY source from the bin-width-weighted transition sums A = (A00, A01, A11),
+ * A_ab = sum_b w_b P_ab:  fr_0 = (A00 s0 + A01 s1 + (W - A00 - A01) s2) / (S W), fr_1 likewise with (A01, A11),
+ * fr_2 = 1 - fr_0 - fr_1.  Equal to the per-bin gfp_mix4 accumulation of gf_bin_loop up to rounding. */
+GF_HD void gfp_transition_fr(const double* A, const gfp_src_consts& c, double* fr) {
+    fr[0] = fma(A[0], c.sd0, fma(A[1], c.sd1, c.ws2)) * c.inv_sw;
+    fr[1] = fma(A[1], c.sd0, fma(A[2], c.sd1, c.ws2)) * c.inv_sw;
+    fr[2] = 1.0 - fr[0] - fr[1];
+}
+
 /* fr_b = sum_i X_bi (sum_a X_ai s_a)  -- NOT divided by sum(s). */
 GF_HD void gfp_mix(const double* X, double s0, double s1, double s2, double* f) {
     const double w0 = fma(X[0], s0, fma(X[3], s1, X[6] * s2));

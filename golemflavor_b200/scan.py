@@ -21,7 +21,7 @@ from .enums import ParamTag, PriorsCateg, Texture, enum_name
 from .param import Param, ParamSet
 
 __all__ = ['sm_paramset', 'scan_paramset', 'scan_model', 'scan_histogram', 'scan_samples', 'ternary_histogram',
-           'shard_range', 'allreduce_counts', 'coverage_mask', 'scan_evidence', 'scan_evidence_grid', 'scan_profile_grid']
+           'shard_range', 'allreduce_counts', 'coverage_mask', 'scan_evidence', 'scan_evidence_grid', 'scan_evidence_sources', 'scan_profile_grid']
 
 DEFAULT_BINNING = np.logspace(np.log10(6e4), np.log10(1e7), 21)  # fr.py:283-285
 
@@ -275,6 +275,92 @@ def scan_evidence_grid(fm, scales, count, seed=26, first_index=0, distributed=Tr
     h = lse.cpu().numpy()
     with np.errstate(divide='ignore'):
         return np.where(h[:, 1] > 0, h[:, 0] + np.log(h[:, 1]) - np.log(count), -np.inf)
+
+
+def source_rows(sources, injected):
+    """Validated ``(sources[nsrc, 3], injected[nsrc, 3])`` float64 arrays for ``scan_evidence_sources``: ``sources`` is one
+    composition ``[3]`` or a list ``[nsrc, 3]``, ``injected`` one composition shared by all sources or one per source.  Every
+    row must be finite and non-negative with a positive sum (it is normalised to unit sum on the device, as ``model.flatten``
+    normalises ``args.source_ratio``).  Raises ValueError otherwise."""
+    src = np.array(sources, dtype=np.float64, ndmin=2)
+    if src.ndim != 2 or src.shape[1] != 3 or src.shape[0] < 1:
+        raise ValueError('sources must be one composition [3] or a list [nsrc, 3], got shape %s' % (np.shape(sources),))
+    inj = np.array(injected, dtype=np.float64, ndmin=2)
+    if inj.ndim != 2 or inj.shape[1] != 3 or inj.shape[0] not in (1, src.shape[0]):
+        raise ValueError('injected must be one composition [3] or one per source [%d, 3], got shape %s' % (src.shape[0], np.shape(injected)))
+    inj = np.ascontiguousarray(np.broadcast_to(inj, src.shape))
+    for name, a in (('source', src), ('injected composition', inj)):
+        bad = ~(np.all(np.isfinite(a) & (a >= 0), axis=1) & (a.sum(axis=1) > 0))
+        if bad.any():
+            j = int(np.nonzero(bad)[0][0])
+            raise ValueError('%s %d = %s: entries must be finite and non-negative with a positive sum' % (name, j, a[j].tolist()))
+    return np.ascontiguousarray(src), inj
+
+
+def _sources_launch(lib, fm, cfg, sc, ns, src, inj, lse, stream):
+    """Enqueue ``gf_scan_evidence_sources`` for ``src`` / ``inj`` (any length: split into calls of at most ``GF_SRC_MAX``)
+    into ``lse`` [nsrc, ns, 2] (a contiguous CUDA tensor)."""
+    torch = _lib.torch_cuda()
+    for j0 in range(0, src.shape[0], _lib.GF_SRC_MAX):
+        s, i = src[j0:j0 + _lib.GF_SRC_MAX], inj[j0:j0 + _lib.GF_SRC_MAX]
+        n = s.shape[0]
+        nbytes = int(lib.gf_scan_evidence_sources_workspace(ns, n))
+        work = _sources_workspace(torch, nbytes)
+        _lib.check(lib.gf_scan_evidence_sources(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, s.ctypes.data_as(C.c_void_p),
+                                                i.ctypes.data_as(C.c_void_p), n, C.c_void_p(lse.data_ptr() + 16 * ns * j0),
+                                                _lib.ptr(work), nbytes, stream))
+
+
+_SRC_WORK = {}
+
+
+def _sources_workspace(torch, nbytes):
+    """Scratch of the source-grid kernel, one buffer per (device, stream), grown on demand and reused by later calls (the
+    kernel leaves it reusable by the next launch on the same stream)."""
+    key = (torch.cuda.current_device(), torch.cuda.current_stream().cuda_stream)
+    buf = _SRC_WORK.get(key)
+    if buf is None or buf.numel() < nbytes:
+        buf = _SRC_WORK[key] = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device='cuda')
+    return buf
+
+
+def _lse_allreduce(dist, lse):
+    """Merge per-rank (max, sum-exp) pairs [..., 2] with two all-reduces: the max, then the sums rescaled to it."""
+    torch = _lib.torch_cuda()
+    gmax = lse[..., 0].clone()
+    dist.all_reduce(gmax, op=dist.ReduceOp.MAX)
+    part = torch.where(torch.isfinite(gmax), lse[..., 1] * torch.exp(lse[..., 0] - gmax), torch.zeros_like(gmax))
+    dist.all_reduce(part, op=dist.ReduceOp.SUM)
+    return torch.stack([gmax, part], dim=-1)
+
+
+def _lnz(h, count):
+    with np.errstate(divide='ignore'):
+        return np.where(h[..., 1] > 0, h[..., 0] + np.log(h[..., 1]) - np.log(count), -np.inf)
+
+
+def scan_evidence_sources(fm, scales, sources, injected, count, seed=26, first_index=0, distributed=True):
+    """``scan_evidence_grid`` for many source compositions at once: ``lnZ[nsrc, len(scales)]``, row j the evidence grid of a
+    model whose source is ``sources[j]`` and whose injected composition is ``injected[j]`` (or the one shared ``injected``
+    [3]).  ONE launch per ``GF_SRC_MAX`` sources (``gf_scan_evidence_sources``): every prior sample is drawn and run through
+    the eigen stage once per scale, then scored for every source.  The model's own source and injected composition are
+    ignored; it must not sample the scale or the source and must have the Gaussian likelihood.  Sharded over ranks and merged
+    like ``scan_evidence_grid``."""
+    src, inj = source_rows(sources, injected)
+    torch = _lib.torch_cuda()
+    dist = _dist() if distributed else None
+    rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
+    start, n = shard_range(count, rank, world, first_index)
+    sc = torch.as_tensor(np.ascontiguousarray(scales, dtype=np.float64).ravel()).cuda()
+    ns = int(sc.numel())
+    lse = torch.empty((src.shape[0], ns, 2), dtype=torch.float64, device='cuda')
+    lse[..., 0] = -np.inf
+    lse[..., 1] = 0.0
+    cfg = _lib.ScanConfig(seed=int(seed), first_index=int(start), count=int(n), nb=0)
+    _sources_launch(_lib.load(), fm, cfg, sc, ns, src, inj, lse, _lib.stream_ptr(torch))
+    if dist and world > 1:
+        lse = _lse_allreduce(dist, lse)
+    return _lnz(lse.cpu().numpy(), count)
 
 
 # defaults of the profile optimiser, from the host-harness study recorded in DESIGN.md (K3c)

@@ -19,9 +19,11 @@ from . import model as _model
 from .enums import ParamTag, Texture
 from .mcmc import DeviceEnsembleSampler
 from .param import Param, ParamSet
-from .scan import DEFAULT_BINNING, PROFILE_NSTARTS, _dist, _profile_launch, shard_range, sm_paramset
+from .scan import (DEFAULT_BINNING, PROFILE_NSTARTS, _dist, _lnz, _lse_allreduce, _profile_launch, _sources_launch, shard_range, sm_paramset,
+                   source_rows)
 
-__all__ = ['scale_grid', 'sweep_paramset', 'sweep', 'evidence_grid', 'profile_grid', 'get_limit', 'limits', 'BAYES_K', 'FREQ_CL']
+__all__ = ['scale_grid', 'sweep_paramset', 'sweep', 'evidence_grid', 'evidence_source_grid', 'profile_grid', 'get_limit', 'limits',
+           'limit_table', 'BAYES_K', 'FREQ_CL']
 
 
 def scale_grid(dimension, segments):
@@ -192,6 +194,43 @@ def _grid_model(dim, texture, src, inj, smearing, binning):
     return _model.flatten(args, None, ParamSet(sm_paramset(with_mass=True)))
 
 
+def evidence_source_grid(sources, dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, injected_ratio=(1, 1, 1),
+                         smearing=0.02, samples=1_000_000, seed=26, binning=DEFAULT_BINNING):
+    """``evidence_grid`` for every source composition of ``sources`` ([nsrc, 3], or one [3]) at once: the reference's
+    submitter runs ``scripts/sens.py`` once per (dimension, texture, source composition, Lambda segment), 30 compositions per
+    texture (``submitter/sens_dag.py:8-16, 38-61, 76-95``).  ``injected_ratio`` is one composition shared by all sources or
+    one per source.  Returns ``{dimension: array[nsrc, segments, 2]}``; ``ev[d][j]`` has exactly the layout of
+    ``evidence_grid(source_ratio=sources[j], injected_ratio=...)[d]`` (the null point -100 and the same scale grid) and the
+    same samples.  ``limit_table`` turns the result into limits.
+
+    ONE launch per dimension (``gf_scan_evidence_sources``; per 256 sources beyond that): the eigen stage of each prior sample
+    runs once per scale, and every source is then scored from its transition sums.  The model of a dimension is built like
+    ``evidence_grid``'s (``_grid_model``); samples are sharded over the ranks of the process group and merged with two
+    all-reduces."""
+    src, inj = source_rows(sources, injected_ratio)
+    torch = _lib.torch_cuda()
+    dist = _dist()
+    rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
+    dims = [int(d) for d in dimensions]
+    grids = [scale_grid(d, segments) for d in dims]
+    nsc = len(grids[0])
+    lse = torch.empty((len(dims), src.shape[0], nsc, 2), dtype=torch.float64, device='cuda')
+    lse[..., 0] = -np.inf
+    lse[..., 1] = 0.0
+    start, n = shard_range(samples, rank, world)
+    cfg = _lib.ScanConfig(seed=int(seed), first_index=int(start), count=int(n), nb=0)
+    lib, stream = _lib.load(), _lib.stream_ptr(torch)
+    scales = torch.as_tensor(np.stack(grids)).cuda()
+    # the model's own source and injected composition are ignored by the kernel: the first row stands in
+    for k, dim in enumerate(dims):
+        fm = _grid_model(dim, texture, src[0], inj[0], smearing, binning)
+        _sources_launch(lib, fm, cfg, scales[k], nsc, src, inj, lse[k], stream)
+    if dist and world > 1:
+        lse = _lse_allreduce(dist, lse)
+    lnz = _lnz(lse.cpu().numpy(), samples)
+    return {d: np.stack([np.broadcast_to(grids[k], lnz[k].shape), lnz[k]], axis=-1) for k, d in enumerate(dims)}
+
+
 def profile_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, source_ratio=(1, 2, 0),
                  injected_ratio=(1, 1, 1), smearing=0.02, nstarts=PROFILE_NSTARTS, seed=27, binning=DEFAULT_BINNING,
                  distributed=True, return_argmax=False):
@@ -318,3 +357,32 @@ def get_limit(scales, statistic, args=None, mask_initial=False, return_interp=Fa
 def limits(evidence, **kwargs):
     """``get_limit`` for every dimension of an ``evidence_grid`` result: ``{dimension: limit or None}``."""
     return {d: get_limit(ev[:, 0], ev[:, 1], **kwargs) for d, ev in evidence.items()}
+
+
+def limit_table(evidence_by_source, **kwargs):
+    """``get_limit`` for every (dimension, source) of an ``evidence_source_grid`` result -- or of any
+    ``{dimension: array[nsrc, segments, 2]}`` of (scale, statistic) curves, e.g. ``profile_grid`` results stacked over sources
+    with ``args=Namespace(stat_method=StatCateg.FREQUENTIST)``: the tabulation of the reference's sensitivities
+    (``plot.plot_table_sens``).  ``kwargs`` go to ``get_limit`` unchanged.  Returns ``(limits[ndims, nsrc],
+    discovered[ndims, nsrc])`` with the dimensions in the dict's order: a limit is NaN where ``get_limit`` returns None or
+    raises 'Discovered LV!', and ``discovered`` is True exactly where it raises 'Discovered LV!'."""
+    dims = list(evidence_by_source)
+    nsrc = {len(evidence_by_source[d]) for d in dims}
+    if len(nsrc) > 1:
+        raise ValueError('limit_table: the dimensions have different numbers of sources: %s' % sorted(nsrc))
+    nsrc = nsrc.pop() if nsrc else 0
+    lim = np.full((len(dims), nsrc), np.nan)
+    disc = np.zeros((len(dims), nsrc), dtype=bool)
+    for i, d in enumerate(dims):
+        for j, ev in enumerate(evidence_by_source[d]):
+            ev = np.asarray(ev, dtype=np.float64)
+            try:
+                v = get_limit(ev[:, 0], ev[:, 1], **kwargs)
+            except AssertionError as e:
+                if str(e) != 'Discovered LV!':
+                    raise
+                disc[i, j] = True
+                continue
+            if v is not None:
+                lim[i, j] = v
+    return lim, disc

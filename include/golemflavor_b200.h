@@ -213,6 +213,25 @@ uint64_t gf_scan_evidence_grid_workspace(int32_t nscales);
 int gf_scan_evidence_grid(const gf_model* model, const gf_scan_config* cfg, const double* d_scales /*[nscales]*/, int32_t nscales,
                           double* d_lse /*[nscales][2]*/, void* d_work, uint64_t work_bytes, void* stream);
 /*
+ * The same grid for many SOURCE COMPOSITIONS in one launch (the reference runs scripts/sens.py once per (dimension, texture,
+ * source composition, Lambda segment), 30 compositions per texture: submitter/sens_dag.py:8-16, 38-61, 76-95).  Each prior
+ * sample is drawn exactly as gf_scan_evidence_grid draws it and its eigen stage is run once per scale; the source enters only
+ * through fr_b = sum_a P_ba s_a with the bin-width-averaged transition P = X X^T of flux_averaged_BSMu (fr.py:441-457), so
+ * every source is then scored at a few instructions.  `sources` and `injected` are HOST arrays [nsrc][3] (source composition
+ * and the injected composition it is scored against; each row normalised to unit sum inside); the model's own fixed_src and
+ * fr_bf are ignored.  d_lse[j][s][0..1] accumulates (max ln L, sum exp) of source j at scale d_scales[s] exactly like
+ * gf_scan_evidence_grid (initialise to {-inf, 0}; the values already there are merged).  d_work is scratch of at least
+ * gf_scan_evidence_sources_workspace(nscales, nsrc) bytes (any contents; reusable by the next call on the same stream).
+ * GF_ERR_ARG, with nothing enqueued, for: a null pointer; nscales outside [1, 65535]; nsrc outside [1, GF_SRC_MAX = 256];
+ * a sampled scale (col_scale >= 0); no_bsm; a sampled source (col_src / col_x / col_src3); llh_kind other than
+ * GF_LLH_GAUSSIAN; a source or injected row with a negative or non-finite entry or a zero sum; a workspace too small.
+ * cfg->count = 0 is a no-op.  The result is the same for any order of the sources (row j depends on row j's compositions only).
+ */
+uint64_t gf_scan_evidence_sources_workspace(int32_t nscales, int32_t nsrc);
+int gf_scan_evidence_sources(const gf_model* model, const gf_scan_config* cfg, const double* d_scales /*[nscales]*/, int32_t nscales,
+                             const double* sources /*HOST [nsrc][3]*/, const double* injected /*HOST [nsrc][3]*/, int32_t nsrc,
+                             double* d_lse /*[nsrc][nscales][2]*/, void* d_work, uint64_t work_bytes, void* stream);
+/*
  * Profile likelihood on the same grid: the frequentist statistic of scripts/sens.py (StatCateg.FREQUENTIST, whose value the
  * reference takes from GolemFit's profiled fit, gf.get_llh_freq / Likelihood.GF_FREQ).  For each frozen scale
  * d_scales[s] = log10(Lambda_s) of a model that does not sample the scale (col_scale = -1), d_best[s] = the maximum of ln_prob
