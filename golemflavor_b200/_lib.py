@@ -12,7 +12,7 @@ import numpy as np
 
 GF_MAX_DIM = 16
 GF_MAX_BINS = 64
-GF_SRC_MAX = 256   # sources per gf_scan_evidence_sources call (csrc/gf_sources_dev.cuh)
+GF_SRC_MAX = 256   # sources per gf_scan_evidence_sources / gf_profile_sources call (csrc/gf_sources_dev.cuh)
 
 GF_OK, GF_ERR_ARG, GF_ERR_CUDA = 0, 1, 2
 ST_OUT_OF_PRIOR, ST_NON_UNITARY, ST_NON_FINITE, ST_ILL_COND, ST_REFINED = 1, 2, 4, 8, 16
@@ -111,6 +111,7 @@ _SIGNATURES = {
     'gf_scan_evidence_sources': (C.c_int, [C.POINTER(Model), C.POINTER(ScanConfig), _P, C.c_int32, _P, _P, C.c_int32, _P, _P, C.c_uint64,
                                            _P]),
     'gf_profile_grid': (C.c_int, [C.POINTER(Model), C.POINTER(ProfileConfig), _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
+    'gf_profile_sources': (C.c_int, [C.POINTER(Model), C.POINTER(ProfileConfig), _P, C.c_int32, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
     'gf_coverage_mask': (C.c_int, [_P, C.c_int64, C.c_double, _P, C.POINTER(C.c_uint64), _P]),
     'gf_hist_smooth': (C.c_int, [_P, C.c_int32, C.c_uint64, _P, C.c_int32, _P, _P, _P]),
     'gf_coverage_mask_f64': (C.c_int, [_P, C.c_int64, C.c_double, _P, C.POINTER(C.c_double), C.POINTER(C.c_uint64), _P]),

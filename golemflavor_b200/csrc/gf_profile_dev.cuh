@@ -1,6 +1,7 @@
 /*
  * gf_profile_dev.cuh -- the profile likelihood of one (scale, start) task: bounded Nelder-Mead over the nuisance
- * parameters of a model whose new-physics scale is frozen (see gf_profile_grid in the C header and gf_profile.cu).
+ * parameters of a model whose new-physics scale is frozen (see gf_profile_grid and gf_profile_sources in the C header and
+ * gf_profile.cu).
  *
  * The optimiser core is templated on the objective, so the host harness runs it on an analytic function as well
  * as on the model.  It is written as a STATE MACHINE that makes exactly one objective evaluation per iteration:
@@ -12,6 +13,7 @@
 #define GF_PROFILE_DEV_CUH
 
 #include "gf_ensemble_dev.cuh" /* GF_*_RN, gf_draw_theta */
+#include "gf_sources_dev.cuh"  /* gf_src_rec, gf_src_llh */
 
 /* the starting simplex: vertex j = x0 + GF_NM_STEP e_(j-1) in scaled coordinates (one sigma of a Gaussian prior, a tenth of a
  * uniform box), stepping inwards when the outward step would leave the box */
@@ -194,6 +196,35 @@ GF_HD double gf_profile_nominal(const gf_dev_model& m, int k) {
     return fmin(fmax(m.mu[k], m.lo[k]), m.hi[k]);
 }
 
+/* The point of the physics at theta: the layout of sens.py for STATIC6 (columns 0-3 mixing coordinates, 4-5 mass
+ * splittings), the model's column map otherwise. */
+template <int SPEC, bool STATIC6>
+GF_HD void gf_profile_point(const gf_dev_model& m, const double* th, gf_point& q) {
+    if constexpr (STATIC6) {
+        q.sm[0] = th[0]; q.sm[1] = th[1]; q.sm[2] = th[2]; q.sm[3] = th[3];
+        q.mass[0] = th[4]; q.mass[1] = th[5];
+        q.src_unit = false;
+    } else {
+        gf_resolve_point<SPEC>(m, [&](int k) { return th[k]; }, q);
+    }
+}
+
+/* -ln_prob of an objective at scaled coordinates x: theta_k = x_k unit_k clipped to the prior box; NaN and +inf ln_prob count
+ * as -inf and set GFP_ST_NON_FINITE in obj.st and obj.nonfinite. */
+template <class Obj>
+GF_HD double gf_profile_neg(Obj& obj, const double* x) {
+    constexpr int NDIM = Obj::NDIM;
+    double th[NDIM > 0 ? NDIM : GF_MAX_DIM];
+    for (int k = 0; k < (NDIM > 0 ? NDIM : obj.m.ndim); ++k) th[k] = obj.theta(x[k], k);
+    const double f = obj.lnprob(th);
+    if (f != f || f == INFINITY) {
+        obj.st |= GFP_ST_NON_FINITE;
+        obj.nonfinite |= GFP_ST_NON_FINITE;
+        return INFINITY;
+    }
+    return -f;
+}
+
 /*
  * -ln_prob at log10 Lambda = log10(lam) of a frozen-scale model (col_scale < 0), on scaled coordinates.  The point is
  * theta_k = x_k unit_k clipped to the prior box; ln_prob is llh.ln_prob as gf_point_lnprob computes it, with the scale
@@ -212,22 +243,21 @@ struct gf_profile_obj {
     GF_HD double hi(int k) const { return GF_DIV_RN(m.hi[k], gf_profile_unit(m, k)); }
     GF_HD double theta(double x, int k) const { return fmin(fmax(GF_MUL_RN(x, gf_profile_unit(m, k)), m.lo[k]), m.hi[k]); }
 
-    GF_HD double lnprob(const double* th) {
-        auto get = [&](int k) { return th[k]; };
-        const double lp = gf_point_lnprior<NDIM>(m, get);
-        if (!(lp > -INFINITY)) { /* as gf_point_lnprob */
+    /* ln prior at th; where it is not finite, fr is NaN and st says why (as gf_point_lnprob) */
+    GF_HD double lnprior(const double* th) {
+        const double lp = gf_point_lnprior<NDIM>(m, [&](int k) { return th[k]; });
+        if (!(lp > -INFINITY)) {
             fr[0] = fr[1] = fr[2] = NAN;
             st = (lp != lp) ? (GFP_ST_NON_FINITE | GFP_ST_OUT_OF_PRIOR) : GFP_ST_OUT_OF_PRIOR;
-            return (lp != lp) ? NAN : -INFINITY;
         }
+        return lp;
+    }
+
+    GF_HD double lnprob(const double* th) {
+        const double lp = lnprior(th);
+        if (!(lp > -INFINITY)) return (lp != lp) ? NAN : -INFINITY;
         gf_point q;
-        if constexpr (STATIC6) { /* the layout of sens.py: columns 0-3 mixing coordinates, 4-5 mass splittings */
-            q.sm[0] = th[0]; q.sm[1] = th[1]; q.sm[2] = th[2]; q.sm[3] = th[3];
-            q.mass[0] = th[4]; q.mass[1] = th[5];
-            q.src_unit = false;
-        } else {
-            gf_resolve_point<SPEC>(m, get, q);
-        }
+        gf_profile_point<SPEC, STATIC6>(m, th, q);
         gf_point_fr_scales<SPEC, ILP>(
             m, q, 1, [&](int) { return lam; },
             [&](int, const double* f, unsigned s) {
@@ -238,33 +268,55 @@ struct gf_profile_obj {
         return lp + gf_multi_gaussian(fr, m.fr_bf, m.half_inv_s2, m.lognorm3, m.offset, m.emulate_underflow, m.underflow_logpdf);
     }
 
-    GF_HD double operator()(const double* x) {
-        double th[NDIM > 0 ? NDIM : GF_MAX_DIM];
-        for (int k = 0; k < (NDIM > 0 ? NDIM : m.ndim); ++k) th[k] = theta(x[k], k);
-        const double f = lnprob(th);
-        if (f != f || f == INFINITY) {
-            st |= GFP_ST_NON_FINITE;
-            nonfinite |= GFP_ST_NON_FINITE;
-            return INFINITY;
-        }
-        return -f;
+    GF_HD double operator()(const double* x) { return gf_profile_neg(*this, x); }
+};
+
+/*
+ * The objective of gf_profile_sources: gf_profile_obj with source record *r substituted for the model's source and injected
+ * composition (the Gaussian likelihood only).  The eigen stage gives the transition sums of gf_point_transition_scales
+ * (ns = 1), and r's composition and likelihood follow from them (gf_src_llh).  st carries the bits gf_point_fr_scales sets:
+ * the eigen stage's, NON_UNITARY and NON_FINITE of the composition.
+ */
+template <int SPEC, bool STATIC6, int ILP>
+struct gf_profile_src_obj : gf_profile_obj<SPEC, STATIC6, ILP> {
+    const gf_src_rec* r;
+
+    GF_HD double lnprob(const double* th) {
+        const gf_dev_model& m = this->m;
+        const double lp = this->lnprior(th);
+        if (!(lp > -INFINITY)) return (lp != lp) ? NAN : -INFINITY;
+        gf_point q;
+        gf_profile_point<SPEC, STATIC6>(m, th, q);
+        double ll = NAN;
+        gf_point_transition_scales<SPEC, ILP>(
+            m, q, 1, [&](int) { return this->lam; },
+            [&](int, const double* A, unsigned s) {
+                double* f = this->fr;
+                ll = gf_src_llh(m, *r, A, f);
+                if (!(fmin(f[0], fmin(f[1], f[2])) >= -m.epsilon)) s |= GFP_ST_NON_UNITARY;
+                if (!(fabs(f[0]) + fabs(f[1]) + fabs(f[2]) < 1e300)) s |= GFP_ST_NON_FINITE;
+                this->st = s;
+            });
+        return lp + ll;
     }
+
+    GF_HD double operator()(const double* x) { return gf_profile_neg(*this, x); }
 };
 
 /*
  * One task: start `k` of the scale whose global index is `task` (start 0: the nominal point; start k >= 1: a prior draw of
  * the scans, gf_draw_theta(m, seed, task * nstarts + k)), optimised in place in S (see gf_nm_minimize).  On return
- * obj.fr / obj.st describe the best vertex, whose ln_prob is -S[((n+1) n + out.best) ld].
+ * obj.fr / obj.st describe the best vertex, whose ln_prob is -S[((n+1) n + out.best) ld].  Obj: gf_profile_obj or
+ * gf_profile_src_obj (Obj::NDIM = 6: the static 6-column layout).
  */
-template <int SPEC, bool STATIC6, int ILP>
-GF_HD gf_nm_out gf_profile_task(gf_profile_obj<SPEC, STATIC6, ILP>& obj, uint64_t seed, uint64_t task, int32_t nstarts, int32_t k,
-                                const gf_nm_opts& o, double* S, int ld) {
-    constexpr int NDIM = STATIC6 ? 6 : 0;
+template <class Obj>
+GF_HD gf_nm_out gf_profile_task(Obj& obj, uint64_t seed, uint64_t task, int32_t nstarts, int32_t k, const gf_nm_opts& o, double* S, int ld) {
+    constexpr int NDIM = Obj::NDIM;
     const gf_dev_model& m = obj.m;
     double x0[NDIM > 0 ? NDIM : GF_MAX_DIM];
     if (k == 0) {
         for (int d = 0; d < (NDIM > 0 ? NDIM : m.ndim); ++d) x0[d] = gf_profile_nominal(m, d);
-    } else if constexpr (STATIC6) {
+    } else if constexpr (NDIM == 6) {
         gf_draw_theta<true, 6>(m, seed, task * (uint64_t)nstarts + (uint64_t)k, x0);
     } else {
         gf_draw_theta(m, seed, task * (uint64_t)nstarts + (uint64_t)k, x0);

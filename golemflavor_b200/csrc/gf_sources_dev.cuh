@@ -41,11 +41,15 @@ GF_HD bool gf_src_record(const double* s, const double* inj, double W, gf_src_re
     return true;
 }
 
-/* llh.multi_gaussian of source r's composition from the transition sums A of one (sample, scale) */
-GF_HD double gf_src_llh(const gf_dev_model& m, const gf_src_rec& r, const double* A) {
-    double fr[3];
+/* llh.multi_gaussian of source r's composition fr (written) from the transition sums A of one (sample, scale) */
+GF_HD double gf_src_llh(const gf_dev_model& m, const gf_src_rec& r, const double* A, double* fr) {
     gfp_transition_fr(A, r.c, fr);
     return gf_multi_gaussian(fr, r.bf, m.half_inv_s2, m.lognorm3, m.offset, m.emulate_underflow, m.underflow_logpdf);
+}
+
+GF_HD double gf_src_llh(const gf_dev_model& m, const gf_src_rec& r, const double* A) {
+    double fr[3];
+    return gf_src_llh(m, r, A, fr);
 }
 
 /* running log-sum-exp (max, sum) += one likelihood: the update rule of k_evidence_grid.  NaN and -inf (pdf underflow)

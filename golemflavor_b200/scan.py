@@ -21,7 +21,8 @@ from .enums import ParamTag, PriorsCateg, Texture, enum_name
 from .param import Param, ParamSet
 
 __all__ = ['sm_paramset', 'scan_paramset', 'scan_model', 'scan_histogram', 'scan_samples', 'ternary_histogram',
-           'shard_range', 'allreduce_counts', 'coverage_mask', 'scan_evidence', 'scan_evidence_grid', 'scan_evidence_sources', 'scan_profile_grid']
+           'shard_range', 'allreduce_counts', 'coverage_mask', 'scan_evidence', 'scan_evidence_grid', 'scan_evidence_sources', 'scan_profile_grid',
+           'scan_profile_sources']
 
 DEFAULT_BINNING = np.logspace(np.log10(6e4), np.log10(1e7), 21)  # fr.py:283-285
 
@@ -399,4 +400,39 @@ def _profile_launch(torch, fm, scales, nstarts, seed, task0, max_evals=PROFILE_M
                              xtol=float(xtol))
     _lib.check(_lib.load().gf_profile_grid(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, _lib.ptr(best), _lib.ptr(argmax), _lib.ptr(fr),
                                            _lib.ptr(st), _lib.ptr(counts), _lib.stream_ptr(torch)))
+    return best, argmax, fr, st, counts
+
+
+def scan_profile_sources(fm, scales, sources, injected, nstarts=PROFILE_NSTARTS, seed=27, task0=0, max_evals=PROFILE_MAX_EVALS, ftol=PROFILE_FTOL,
+                         xtol=PROFILE_XTOL):
+    """``scan_profile_grid`` for many source compositions at once: row j is the profile of a model whose source is
+    ``sources[j]`` and whose injected composition is ``injected[j]`` (or the one shared ``injected`` [3]), from the same starts
+    at every scale.  ONE launch per ``GF_SRC_MAX`` sources (``gf_profile_sources``: one block per (scale, source)).  The model's
+    own source and injected composition are ignored; it must not sample the scale or the source and must have the Gaussian
+    likelihood.  Returns the dict of ``scan_profile_grid`` with a leading ``[nsrc]`` axis."""
+    src, inj = source_rows(sources, injected)
+    torch = _lib.torch_cuda()
+    out = _profile_sources_launch(torch, fm, scales, src, inj, nstarts, seed, task0, max_evals, ftol, xtol)
+    best, argmax, fr, st, counts = (t.cpu().numpy() for t in out)
+    return dict(best=best, argmax=argmax, fr=fr, status=st, nevals=counts[..., 0], nconverged=counts[..., 1])
+
+
+def _profile_sources_launch(torch, fm, scales, src, inj, nstarts, seed, task0, max_evals=PROFILE_MAX_EVALS, ftol=PROFILE_FTOL, xtol=PROFILE_XTOL):
+    """Enqueue ``gf_profile_sources`` on torch's current stream for the validated rows ``src`` / ``inj`` (any number: split into
+    calls of at most ``GF_SRC_MAX``): (best, argmax, fr, status, counts) as CUDA tensors with a leading [nsrc] axis."""
+    sc = torch.as_tensor(np.ascontiguousarray(scales, dtype=np.float64).ravel()).cuda()
+    ns, nsrc = int(sc.numel()), src.shape[0]
+    best = torch.empty((nsrc, ns), dtype=torch.float64, device='cuda')
+    argmax = torch.empty((nsrc, ns, fm.ndim), dtype=torch.float64, device='cuda')
+    fr = torch.empty((nsrc, ns, 3), dtype=torch.float64, device='cuda')
+    st = torch.empty((nsrc, ns), dtype=torch.uint8, device='cuda')
+    counts = torch.empty((nsrc, ns, 2), dtype=torch.int64, device='cuda')
+    cfg = _lib.ProfileConfig(seed=int(seed), task0=int(task0), nstarts=int(nstarts), max_evals=int(max_evals), ftol=float(ftol),
+                             xtol=float(xtol))
+    lib, stream = _lib.load(), _lib.stream_ptr(torch)
+    for j0 in range(0, nsrc, _lib.GF_SRC_MAX):
+        s, i = src[j0:j0 + _lib.GF_SRC_MAX], inj[j0:j0 + _lib.GF_SRC_MAX]
+        _lib.check(lib.gf_profile_sources(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, s.ctypes.data_as(C.c_void_p), i.ctypes.data_as(C.c_void_p),
+                                          s.shape[0], _lib.ptr(best[j0]), _lib.ptr(argmax[j0]), _lib.ptr(fr[j0]), _lib.ptr(st[j0]),
+                                          _lib.ptr(counts[j0]), stream))
     return best, argmax, fr, st, counts

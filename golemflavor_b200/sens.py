@@ -19,11 +19,11 @@ from . import model as _model
 from .enums import ParamTag, Texture
 from .mcmc import DeviceEnsembleSampler
 from .param import Param, ParamSet
-from .scan import (DEFAULT_BINNING, PROFILE_NSTARTS, _dist, _lnz, _lse_allreduce, _profile_launch, _sources_launch, shard_range, sm_paramset,
-                   source_rows)
+from .scan import (DEFAULT_BINNING, PROFILE_NSTARTS, _dist, _lnz, _lse_allreduce, _profile_launch, _profile_sources_launch, _sources_launch,
+                   shard_range, sm_paramset, source_rows)
 
-__all__ = ['scale_grid', 'sweep_paramset', 'sweep', 'evidence_grid', 'evidence_source_grid', 'profile_grid', 'get_limit', 'limits',
-           'limit_table', 'BAYES_K', 'FREQ_CL']
+__all__ = ['scale_grid', 'sweep_paramset', 'sweep', 'evidence_grid', 'evidence_source_grid', 'profile_grid', 'profile_source_grid', 'get_limit',
+           'limits', 'limit_table', 'BAYES_K', 'FREQ_CL']
 
 
 def scale_grid(dimension, segments):
@@ -282,6 +282,63 @@ def profile_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OE
     return prof
 
 
+def profile_source_grid(sources, dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, injected_ratio=(1, 1, 1), smearing=0.02,
+                        nstarts=PROFILE_NSTARTS, seed=27, binning=DEFAULT_BINNING, distributed=True, return_argmax=False):
+    """``profile_grid`` for every source composition of ``sources`` ([nsrc, 3], or one [3]) at once: the frequentist column of the
+    reference's sensitivity table, whose submitter runs ``scripts/sens.py`` once per (dimension, texture, source composition,
+    Lambda segment), 30 compositions per texture (``submitter/sens_dag.py``).  ``injected_ratio`` is one composition shared by
+    all sources or one per source.  Returns ``{dimension: array[nsrc, segments, 2]}`` of (scale, profile ln_prob), the layout
+    of ``evidence_source_grid``: ``limit_table(result, args=Namespace(stat_method=StatCateg.FREQUENTIST))`` gives the frequentist
+    table.  Every source starts from the points ``profile_grid`` uses at each scale.  With ``return_argmax`` also
+    ``{dimension: array[nsrc, segments, 6]}`` of the maximising parameters.
+
+    ONE launch per dimension (per 256 sources beyond that; ``gf_profile_sources``: one block per (scale, source), one thread per
+    start), on one stream per dimension, with the model of ``_grid_model``.  The (dimension, scale) rows are sharded over the
+    ranks of the process group exactly as ``profile_grid`` shards them, and the disjoint rows are merged with one all-reduce:
+    the result is the same for any number of ranks."""
+    src, inj = source_rows(sources, injected_ratio)
+    torch = _lib.torch_cuda()
+    dist = _dist() if distributed else None
+    rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
+    dims = [int(d) for d in dimensions]
+    segments = int(segments)
+    nsrc = src.shape[0]
+    grid = [(k, s) for k in range(len(dims)) for s in range(segments)]
+    start, count = shard_range(len(grid), rank, world)
+    ndim = len(sm_paramset(with_mass=True))
+    rows = np.zeros((len(grid), nsrc, 1 + ndim))
+    cur = torch.cuda.current_stream()
+    pending = []
+    # the model's own source and injected composition are ignored by the kernel: the first row stands in
+    for k, dim in enumerate(dims):
+        mine = [s for kk, s in grid[start:start + count] if kk == k]
+        if not mine:
+            continue
+        fm = _grid_model(dim, texture, src[0], inj[0], smearing, binning)
+        scales = scale_grid(dim, segments)[mine[0]:mine[-1] + 1]
+        stream = _dim_stream(torch, dim)
+        stream.wait_stream(cur)
+        with torch.cuda.stream(stream):
+            out = _profile_sources_launch(torch, fm, scales, src, inj, nstarts, seed, mine[0])
+        pending.append((stream, k * segments + mine[0], out))
+    for stream, row0, (best, argmax, _, _, _) in pending:
+        stream.synchronize()
+        n = best.shape[1]
+        rows[row0:row0 + n, :, 0] = best.cpu().numpy().T
+        rows[row0:row0 + n, :, 1:] = argmax.cpu().numpy().transpose(1, 0, 2)
+    if dist and world > 1:
+        t = torch.as_tensor(rows).cuda()
+        dist.all_reduce(t, op=dist.ReduceOp.SUM)                   # disjoint rows: sum == gather
+        rows = t.cpu().numpy()
+    prof = {}
+    for k, d in enumerate(dims):
+        r = rows[k * segments:(k + 1) * segments].transpose(1, 0, 2)          # [nsrc, segments, 1 + ndim]
+        prof[d] = np.stack([np.broadcast_to(scale_grid(d, segments), r.shape[:2]), r[..., 0]], axis=-1)
+    if return_argmax:
+        return prof, {d: rows[k * segments:(k + 1) * segments, :, 1:].transpose(1, 0, 2).copy() for k, d in enumerate(dims)}
+    return prof
+
+
 _WORK = {}
 
 
@@ -361,8 +418,8 @@ def limits(evidence, **kwargs):
 
 def limit_table(evidence_by_source, **kwargs):
     """``get_limit`` for every (dimension, source) of an ``evidence_source_grid`` result -- or of any
-    ``{dimension: array[nsrc, segments, 2]}`` of (scale, statistic) curves, e.g. ``profile_grid`` results stacked over sources
-    with ``args=Namespace(stat_method=StatCateg.FREQUENTIST)``: the tabulation of the reference's sensitivities
+    ``{dimension: array[nsrc, segments, 2]}`` of (scale, statistic) curves, e.g. of ``profile_source_grid`` with
+    ``args=Namespace(stat_method=StatCateg.FREQUENTIST)``: the tabulation of the reference's sensitivities
     (``plot.plot_table_sens``).  ``kwargs`` go to ``get_limit`` unchanged.  Returns ``(limits[ndims, nsrc],
     discovered[ndims, nsrc])`` with the dimensions in the dict's order: a limit is NaN where ``get_limit`` returns None or
     raises 'Discovered LV!', and ``discovered`` is True exactly where it raises 'Discovered LV!'."""

@@ -259,6 +259,29 @@ int gf_profile_grid(const gf_model* model, const gf_profile_config* cfg, const d
                     double* d_best /*[nscales]*/, double* d_argmax /*[nscales][ndim] or NULL*/,
                     double* d_fr /*[nscales][3] or NULL*/, uint8_t* d_status /*[nscales] or NULL*/,
                     int64_t* d_counts /*[nscales][2] or NULL: evaluations, starts that converged*/, void* stream);
+/*
+ * The profile likelihood for many SOURCE COMPOSITIONS in one launch: the frequentist column of the reference's sensitivity
+ * table (scripts/sens.py with StatCateg.FREQUENTIST, run once per source composition, 30 per texture: submitter/sens_dag.py).
+ * Row (j, s) is gf_profile_grid's task with source j: d_best[j][s] = the maximum over the model's columns inside their prior
+ * box of ln_prob at log10 Lambda = d_scales[s], with sources[j] as the source composition and injected[j] as the injected
+ * composition the Gaussian likelihood scores it against.  `sources` and `injected` are HOST arrays [nsrc][3], each row
+ * normalised to unit sum inside; the model's own fixed_src and fr_bf are ignored.  The composition comes from the eigen
+ * stage's transition sums (as gf_scan_evidence_sources), which differ from gf_profile_grid's per-bin mix in rounding only.
+ * The optimiser, the starts and the configuration are gf_profile_grid's: start 0 = the nominal point, start k >= 1 = the prior
+ * draw with sample index (task0 + s) * nstarts + k for every source, the best start wins (ties: the lower k).  A row
+ * therefore depends on (seed, task0 + s, nstarts, source j, injected j) only: not on the other sources, their order, or how
+ * the scales are split over calls or GPUs.  Optional outputs as gf_profile_grid's, per row: d_argmax[j][s], d_fr[j][s],
+ * d_status[j][s], d_counts[j][s].  One launch: one block per (scale, source), one thread per start.
+ * GF_ERR_ARG, with nothing enqueued, for: a null pointer; nscales outside [0, 2^30]; nsrc outside [1, GF_SRC_MAX = 256];
+ * a sampled scale; no_bsm; a sampled source; llh_kind other than GF_LLH_GAUSSIAN; a source or injected row with a negative or
+ * non-finite entry or a zero sum; nstarts not a multiple of 32 in [32, 256]; max_evals < 1; ftol or xtol negative;
+ * task0 < 0; a uniform prior without a finite box; simplices that do not fit in shared memory.  nscales = 0 is a no-op.
+ */
+int gf_profile_sources(const gf_model* model, const gf_profile_config* cfg, const double* d_scales /*[nscales]*/, int32_t nscales,
+                       const double* sources /*HOST [nsrc][3]*/, const double* injected /*HOST [nsrc][3]*/, int32_t nsrc,
+                       double* d_best /*[nsrc][nscales]*/, double* d_argmax /*[nsrc][nscales][ndim] or NULL*/,
+                       double* d_fr /*[nsrc][nscales][3] or NULL*/, uint8_t* d_status /*[nsrc][nscales] or NULL*/,
+                       int64_t* d_counts /*[nsrc][nscales][2] or NULL*/, void* stream);
 /* Highest-density coverage region of a histogram (plot.flavor_contour, plot.py:372-384: normalise,
  * sort cells by content, cumulative sum, `thres = searchsorted(cumsum, coverage/100)`, mask the first
  * `thres` cells).  d_mask[i] = 1 for the cells inside the region.  h_info (host, optional) receives
