@@ -43,4 +43,17 @@ int gf_build_dev_model(const gf_model* m, gf_dev_model* d);
 /* number of SMs of the current device (cached) */
 int gf_sm_count(int* sms);
 
+/* The refusals of every frozen-scale grid entry point `who`: the model needs a BSM path and must not sample the scale. */
+int gf_check_frozen_scale(const char* who, const gf_dev_model& d);
+
+/* Blocks in x of an evidence-grid launch of ny scale groups: as many as fit the device in ONE wave at per_sm blocks per
+ * SM (every block carries the same amount of work, so blocks left for a second wave would double the time), no more than
+ * the samples need, at least one. */
+unsigned gf_evidence_nx(int sms, int per_sm, int ny, uint64_t count, int threads);
+
+/* The workspace of an evidence-grid launch: per-block partials [rows][nx][2], then one ticket per scale group (ny), cleared
+ * on stream st.  Refuses a workspace smaller than that (`who`_workspace gives its size). */
+int gf_evidence_workspace(const char* who, size_t rows, unsigned nx, int ny, void* d_work, uint64_t work_bytes, cudaStream_t st, double** part,
+                          unsigned int** tickets);
+
 #endif /* GF_COMMON_CUH */

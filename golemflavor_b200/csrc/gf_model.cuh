@@ -119,6 +119,7 @@ GF_HD bool gf_model_is_fixed_spec(const gf_dev_model& m);
 GF_HD bool gf_model_has_fixed_source(const gf_dev_model& m);
 GF_HD int gf_model_spec(const gf_dev_model& m);
 GF_HD int gf_model_layout_spec(const gf_dev_model& m);
+GF_HD int gf_model_grid_spec(const gf_dev_model& m);
 
 /* the general case: runtime column map */
 template <int SPEC, class Get>
@@ -594,6 +595,11 @@ GF_HD bool gf_model_has_fixed_source(const gf_dev_model& m) { return m.col_src[0
 
 GF_HD bool gf_model_is_fixed_spec(const gf_dev_model& m) { return !m.no_bsm && !m.np_free && gf_model_has_fixed_source(m); }
 
+/* columns 0-3 the mixing coordinates, 4-5 the mass splittings: the head of the layout of sens.py */
+GF_HD bool gf_model_has_head6(const gf_dev_model& m) {
+    return m.col_sm[0] == 0 && m.col_sm[1] == 1 && m.col_sm[2] == 2 && m.col_sm[3] == 3 && m.col_mass[0] == 4 && m.col_mass[1] == 5;
+}
+
 /* the specialisation a model's COLUMN LAYOUT allows (kernels without a GF_SPEC_NPFREE instance map it to GF_SPEC_GENERIC) */
 GF_HD int gf_model_layout_spec(const gf_dev_model& m) {
     if (m.no_bsm) {
@@ -603,10 +609,17 @@ GF_HD int gf_model_layout_spec(const gf_dev_model& m) {
     }
     if (!gf_model_has_fixed_source(m)) return GF_SPEC_GENERIC;
     if (m.np_free) return GF_SPEC_NPFREE;
-    const bool head = m.col_sm[0] == 0 && m.col_sm[1] == 1 && m.col_sm[2] == 2 && m.col_sm[3] == 3 && m.col_mass[0] == 4 && m.col_mass[1] == 5;
+    const bool head = gf_model_has_head6(m);
     if (head && m.ndim == 7 && m.col_scale == 6) return GF_SPEC_FIXED7;
     if (head && m.ndim == 12 && m.col_scale == 11) return GF_SPEC_FIXED12;
     return GF_SPEC_FIXED;
+}
+
+/* which instance the frozen-scale grid kernels (k_evidence_grid, k_evidence_sources, k_profile, k_profile_sources) launch:
+ * 2 = <GF_SPEC_FIXED, STATIC6> for the six columns of sens.py, 1 = <GF_SPEC_FIXED, false>, 0 = <GF_SPEC_GENERIC, false> */
+GF_HD int gf_model_grid_spec(const gf_dev_model& m) {
+    const bool fixed = gf_model_is_fixed_spec(m);
+    return fixed && m.ndim == 6 && gf_model_has_head6(m) ? 2 : fixed ? 1 : 0;
 }
 
 /* which specialisation the log-posterior and sampler kernels launch: the layout's, unless it also fixes the prior kinds at

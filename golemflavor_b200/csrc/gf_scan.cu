@@ -592,18 +592,6 @@ extern "C" int gf_coverage_mask_f64(const double* d_field, int64_t cells, double
 
 /* ------------------------------------------------------------------ Monte-Carlo evidence */
 
-__device__ __forceinline__ void gf_lse_merge(double& m, double& s, double m2, double s2) {
-    /* (m, s) <- log-sum-exp merge of two partials; empty partials are (-inf, 0) */
-    const double mm = fmax(m, m2);
-    if (mm == -INFINITY) {
-        m = -INFINITY;
-        s = 0.0;
-        return;
-    }
-    s = s * exp(m - mm) + s2 * exp(m2 - mm);
-    m = mm;
-}
-
 template <int SPEC>
 __global__ void __launch_bounds__(GF_SCAN_THREADS, GF_SCAN_MIN_BLOCKS)
     k_evidence(const __grid_constant__ gf_dev_model m, const uint64_t seed, const uint64_t first_index, const uint64_t count,
@@ -723,16 +711,9 @@ __global__ void __launch_bounds__(GF_SCAN_THREADS, GF_SCAN_MIN_BLOCKS)
                 const double ll = m.llh_kind == GF_LLH_FLAT
                                       ? m.llh_const
                                       : gf_multi_gaussian(fr, m.fr_bf, m.half_inv_s2, m.lognorm3, m.offset, m.emulate_underflow, m.underflow_logpdf);
-                if (ll > -INFINITY) { /* NaN and -inf (pdf underflow) carry no weight */
+                if (ll > -INFINITY) { /* only the samples with weight touch shared memory */
                     double mo = sh_m[k * T + tid], so = sh_s[k * T + tid];
-                    const double d = ll - mo;        /* +inf on the first sample */
-                    const double e = exp(-fabs(d));
-                    if (d <= 0.0) {
-                        so += e;
-                    } else {
-                        so = fma(so, e, 1.0);
-                        mo = ll;
-                    }
+                    gf_lse_push(mo, so, ll);
                     sh_m[k * T + tid] = mo;
                     sh_s[k * T + tid] = so;
                 }
@@ -797,17 +778,37 @@ int evg_plan(K kern, int nscales, uint64_t count, evg_geometry* geo) {
     GF_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, GF_SCAN_THREADS, smem));
     GF_REQUIRE(per_sm >= 1, "gf_scan_evidence_grid: kernel does not fit on an SM (smem %zu B)", smem);
     const int ny = (nscales + s_per - 1) / s_per;
-    const uint64_t want = (count + GF_SCAN_THREADS - 1) / GF_SCAN_THREADS;
-    /* every block carries the same amount of work: the grid must fit the device in ONE wave (rounding the x extent up
-     * would leave a few blocks for a second wave that takes as long as the first) */
-    uint64_t nx = ((uint64_t)sms * per_sm) / ny;
-    if (nx > want) nx = want;
-    if (nx < 1) nx = 1;
-    geo->s_per = s_per; geo->ny = ny; geo->per_sm = per_sm; geo->nx = (unsigned)nx; geo->smem = smem;
+    geo->s_per = s_per; geo->ny = ny; geo->per_sm = per_sm; geo->nx = gf_evidence_nx(sms, per_sm, ny, count, GF_SCAN_THREADS); geo->smem = smem;
     return GF_OK;
 }
 
 }  // namespace
+
+int gf_check_frozen_scale(const char* who, const gf_dev_model& d) {
+    GF_REQUIRE(!d.no_bsm, "%s: the model has no BSM path (no_bsm = 1)", who);
+    GF_REQUIRE(d.col_scale < 0, "%s: the scale must not be a sampled column (col_scale = %d): it is frozen at the grid values", who, d.col_scale);
+    return GF_OK;
+}
+
+unsigned gf_evidence_nx(int sms, int per_sm, int ny, uint64_t count, int threads) {
+    const uint64_t want = (count + threads - 1) / threads;
+    uint64_t nx = ((uint64_t)sms * per_sm) / ny;
+    if (nx > want) nx = want;
+    if (nx < 1) nx = 1;
+    return (unsigned)nx;
+}
+
+int gf_evidence_workspace(const char* who, size_t rows, unsigned nx, int ny, void* d_work, uint64_t work_bytes, cudaStream_t st, double** part,
+                          unsigned int** tickets) {
+    const size_t part_bytes = rows * nx * 2 * sizeof(double);
+    const size_t need = part_bytes + (size_t)ny * sizeof(unsigned int);
+    GF_REQUIRE(d_work != nullptr && work_bytes >= need, "%s: workspace of %llu B is too small, need %llu B (%s_workspace)", who,
+               (unsigned long long)work_bytes, (unsigned long long)need, who);
+    *part = static_cast<double*>(d_work);
+    *tickets = reinterpret_cast<unsigned int*>(static_cast<char*>(d_work) + part_bytes);
+    GF_CUDA(cudaMemsetAsync(*tickets, 0, (size_t)ny * sizeof(unsigned int), st));
+    return GF_OK;
+}
 
 extern "C" uint64_t gf_scan_evidence_grid_workspace(int32_t nscales) {
     int sms = 0;
@@ -822,23 +823,16 @@ extern "C" int gf_scan_evidence_grid(const gf_model* model, const gf_scan_config
     GF_REQUIRE(nscales >= 1 && nscales <= 65535, "gf_scan_evidence_grid: nscales = %d outside [1, 65535]", nscales);
     gf_dev_model d;
     if (int rc = gf_build_dev_model(model, &d)) return rc;
-    GF_REQUIRE(!d.no_bsm, "gf_scan_evidence_grid: the model has no BSM path (no_bsm = 1)");
-    GF_REQUIRE(d.col_scale < 0, "gf_scan_evidence_grid: the scale must not be a sampled column (col_scale = %d): it is frozen at the grid values", d.col_scale);
+    if (int rc = gf_check_frozen_scale("gf_scan_evidence_grid", d)) return rc;
     if (cfg->count == 0) return GF_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    const bool fixed = gf_model_is_fixed_spec(d);
-    const bool static6 = fixed && d.ndim == 6 && d.col_sm[0] == 0 && d.col_sm[1] == 1 && d.col_sm[2] == 2 && d.col_sm[3] == 3 &&
-                         d.col_mass[0] == 4 && d.col_mass[1] == 5;
-    auto kern = static6 ? k_evidence_grid<GF_SPEC_FIXED, true> : fixed ? k_evidence_grid<GF_SPEC_FIXED, false> : k_evidence_grid<GF_SPEC_GENERIC, false>;
+    const int spec = gf_model_grid_spec(d);
+    auto kern = spec == 2 ? k_evidence_grid<GF_SPEC_FIXED, true> : spec == 1 ? k_evidence_grid<GF_SPEC_FIXED, false> : k_evidence_grid<GF_SPEC_GENERIC, false>;
     evg_geometry geo;
     if (int rc = evg_plan(kern, nscales, cfg->count, &geo)) return rc;
-    const size_t part_bytes = (size_t)nscales * geo.nx * 2 * sizeof(double);
-    const size_t need = part_bytes + (size_t)geo.ny * sizeof(unsigned int);
-    GF_REQUIRE(d_work != nullptr && work_bytes >= need, "gf_scan_evidence_grid: workspace of %llu B is too small, need %llu B (gf_scan_evidence_grid_workspace)",
-               (unsigned long long)work_bytes, (unsigned long long)need);
-    double* part = static_cast<double*>(d_work);
-    unsigned int* tickets = reinterpret_cast<unsigned int*>(static_cast<char*>(d_work) + part_bytes);
-    GF_CUDA(cudaMemsetAsync(tickets, 0, (size_t)geo.ny * sizeof(unsigned int), st));
+    double* part = nullptr;
+    unsigned int* tickets = nullptr;
+    if (int rc = gf_evidence_workspace("gf_scan_evidence_grid", nscales, geo.nx, geo.ny, d_work, work_bytes, st, &part, &tickets)) return rc;
     kern<<<dim3(geo.nx, (unsigned)geo.ny), GF_SCAN_THREADS, geo.smem, st>>>(d, cfg->seed, cfg->first_index, cfg->count, d_scales, nscales, geo.s_per, part,
                                                                               tickets, d_lse);
     ++g_gf_launches;

@@ -73,7 +73,7 @@ __global__ void __launch_bounds__(GF_EVS_THREADS, GF_EVS_MIN_BLOCKS)
             double mq = acc[(2 * q) * T + tid], sq = acc[(2 * q + 1) * T + tid];
             for (int t = t0; t < t0 + L; ++t) {
                 const double A[3] = {a[t], a[T + t], a[2 * T + t]};
-                gf_src_lse_push(mq, sq, gf_src_llh(m, r, A)); /* a NaN marker gives a NaN likelihood: no weight */
+                gf_lse_push(mq, sq, gf_src_llh(m, r, A)); /* a NaN marker gives a NaN likelihood: no weight */
             }
             acc[(2 * q) * T + tid] = mq;
             acc[(2 * q + 1) * T + tid] = sq;
@@ -85,7 +85,7 @@ __global__ void __launch_bounds__(GF_EVS_THREADS, GF_EVS_MIN_BLOCKS)
     for (int pair = tid; pair < npairs; pair += T) {
         const int u = pair * G, q = u / T, t = u - q * T;
         double mx = acc[(2 * q) * T + t], sm = acc[(2 * q + 1) * T + t];
-        for (int c = 1; c < G; ++c) gf_src_lse_merge(mx, sm, acc[t + c], acc[T + t + c]);
+        for (int c = 1; c < G; ++c) gf_lse_merge(mx, sm, acc[t + c], acc[T + t + c]);
         double* o = partials + 2 * (((size_t)(s0 + pair / nsrc) * nsrc + pair % nsrc) * nx + blockIdx.x);
         o[0] = mx;
         o[1] = sm;
@@ -102,7 +102,7 @@ __global__ void __launch_bounds__(GF_EVS_THREADS, GF_EVS_MIN_BLOCKS)
         double* dst = lse + 2 * ((size_t)j * nscales + s0 + k);
         double mx = dst[0], sm = dst[1];
         const volatile double* in = partials + 2 * ((size_t)(s0 + k) * nsrc + j) * nx;
-        for (unsigned b = 0; b < gridDim.x; ++b) gf_src_lse_merge(mx, sm, in[2 * b], in[2 * b + 1]); /* block order */
+        for (unsigned b = 0; b < gridDim.x; ++b) gf_lse_merge(mx, sm, in[2 * b], in[2 * b + 1]); /* block order */
         dst[0] = mx;
         dst[1] = sm;
     }
@@ -145,6 +145,19 @@ size_t evs_smem(const evs_plan_t& p) { return (size_t)(GF_EVS_MAX_S_PER + (2 * p
 
 }  // namespace
 
+int gf_src_table_fill(const char* who, const gf_dev_model& d, const double* sources, const double* injected, int nsrc, gf_src_table* S) {
+    GF_REQUIRE(gf_model_has_fixed_source(d), "%s: the model samples the source (col_src / col_x / col_src3): the sources are the launch's own list",
+               who);
+    GF_REQUIRE(d.llh_kind == GF_LLH_GAUSSIAN, "%s: llh_kind = %d, the Gaussian likelihood (GF_LLH_GAUSSIAN) is required", who, d.llh_kind);
+    S->nsrc = nsrc;
+    S->reserved = 0;
+    for (int j = 0; j < nsrc; ++j)
+        GF_REQUIRE(gf_src_record(sources + 3 * j, injected + 3 * j, d.wsum, &S->src[j]),
+                   "%s: source %d = (%g, %g, %g) / injected (%g, %g, %g): entries must be finite and non-negative with a positive sum", who, j,
+                   sources[3 * j], sources[3 * j + 1], sources[3 * j + 2], injected[3 * j], injected[3 * j + 1], injected[3 * j + 2]);
+    return GF_OK;
+}
+
 extern "C" uint64_t gf_scan_evidence_sources_workspace(int32_t nscales, int32_t nsrc) {
     int sms = 0;
     if (nscales < 1 || nscales > 65535 || nsrc < 1 || nsrc > GF_SRC_MAX || gf_sm_count(&sms) != GF_OK) return 0;
@@ -164,53 +177,30 @@ extern "C" int gf_scan_evidence_sources(const gf_model* model, const gf_scan_con
     GF_REQUIRE(nsrc >= 1 && nsrc <= GF_SRC_MAX, "gf_scan_evidence_sources: nsrc = %d outside [1, %d]", nsrc, GF_SRC_MAX);
     gf_dev_model d;
     if (int rc = gf_build_dev_model(model, &d)) return rc;
-    GF_REQUIRE(!d.no_bsm, "gf_scan_evidence_sources: the model has no BSM path (no_bsm = 1)");
-    GF_REQUIRE(d.col_scale < 0, "gf_scan_evidence_sources: the scale must not be a sampled column (col_scale = %d): it is frozen at the grid values",
-               d.col_scale);
-    GF_REQUIRE(gf_model_has_fixed_source(d), "gf_scan_evidence_sources: the model samples the source (col_src / col_x / col_src3): the sources are "
-               "the launch's own list");
-    GF_REQUIRE(d.llh_kind == GF_LLH_GAUSSIAN, "gf_scan_evidence_sources: llh_kind = %d, the Gaussian likelihood (GF_LLH_GAUSSIAN) is required",
-               d.llh_kind);
+    if (int rc = gf_check_frozen_scale("gf_scan_evidence_sources", d)) return rc;
     gf_src_table tab; /* 14 KB, copied into the kernel parameter buffer by the launch */
-    gf_src_table* S = &tab;
-    S->nsrc = nsrc;
-    S->reserved = 0;
-    for (int j = 0; j < nsrc; ++j)
-        GF_REQUIRE(gf_src_record(sources + 3 * j, injected + 3 * j, d.wsum, &S->src[j]),
-                   "gf_scan_evidence_sources: source %d = (%g, %g, %g) / injected (%g, %g, %g): entries must be finite and non-negative with a "
-                   "positive sum",
-                   j, sources[3 * j], sources[3 * j + 1], sources[3 * j + 2], injected[3 * j], injected[3 * j + 1], injected[3 * j + 2]);
+    if (int rc = gf_src_table_fill("gf_scan_evidence_sources", d, sources, injected, nsrc, &tab)) return rc;
     const evs_plan_t p = evs_plan(nscales, nsrc);
-    const bool fixed = gf_model_is_fixed_spec(d);
-    const bool static6 = fixed && d.ndim == 6 && d.col_sm[0] == 0 && d.col_sm[1] == 1 && d.col_sm[2] == 2 && d.col_sm[3] == 3 &&
-                         d.col_mass[0] == 4 && d.col_mass[1] == 5;
-    auto kern = static6 ? k_evidence_sources<GF_SPEC_FIXED, true> : fixed ? k_evidence_sources<GF_SPEC_FIXED, false> : k_evidence_sources<GF_SPEC_GENERIC, false>;
+    const int spec = gf_model_grid_spec(d);
+    auto kern = spec == 2 ? k_evidence_sources<GF_SPEC_FIXED, true> : spec == 1 ? k_evidence_sources<GF_SPEC_FIXED, false>
+                                                                                : k_evidence_sources<GF_SPEC_GENERIC, false>;
     const size_t smem = evs_smem(p);
     int sms = 0;
     if (int rc = gf_sm_count(&sms)) return rc;
     if (cfg->count == 0) return GF_OK;
-    const uint64_t want = (cfg->count + GF_EVS_THREADS - 1) / GF_EVS_THREADS;
-    const uint64_t cap = (uint64_t)sms * EVS_MAX_BLOCKS_PER_SM / (uint64_t)p.ny;
     GF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 1;
     GF_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, GF_EVS_THREADS, smem));
     GF_REQUIRE(per_sm >= 1, "gf_scan_evidence_sources: kernel does not fit on an SM (smem %zu B)", smem);
-    /* one wave: every block carries the same amount of work */
-    uint64_t nx = ((uint64_t)sms * (uint64_t)(per_sm < EVS_MAX_BLOCKS_PER_SM ? per_sm : EVS_MAX_BLOCKS_PER_SM)) / (uint64_t)p.ny;
-    if (nx > want) nx = want;
-    if (nx > cap) nx = cap;
-    if (nx < 1) nx = 1;
-    const size_t part_bytes = (size_t)nscales * nsrc * nx * 2 * sizeof(double);
-    const size_t need = part_bytes + (size_t)p.ny * sizeof(unsigned int);
-    GF_REQUIRE(d_work != nullptr && work_bytes >= need,
-               "gf_scan_evidence_sources: workspace of %llu B is too small, need %llu B (gf_scan_evidence_sources_workspace)",
-               (unsigned long long)work_bytes, (unsigned long long)need);
+    /* the workspace holds EVS_MAX_BLOCKS_PER_SM blocks per SM */
+    const unsigned nx = gf_evidence_nx(sms, per_sm < EVS_MAX_BLOCKS_PER_SM ? per_sm : EVS_MAX_BLOCKS_PER_SM, p.ny, cfg->count, GF_EVS_THREADS);
     cudaStream_t st = (cudaStream_t)stream;
-    double* part = static_cast<double*>(d_work);
-    unsigned int* tickets = reinterpret_cast<unsigned int*>(static_cast<char*>(d_work) + part_bytes);
-    GF_CUDA(cudaMemsetAsync(tickets, 0, (size_t)p.ny * sizeof(unsigned int), st));
-    kern<<<dim3((unsigned)nx, (unsigned)p.ny), GF_EVS_THREADS, smem, st>>>(d, *S, cfg->seed, cfg->first_index, cfg->count, d_scales, nscales,
-                                                                            p.s_per, p.G, p.slots, part, tickets, d_lse);
+    double* part = nullptr;
+    unsigned int* tickets = nullptr;
+    if (int rc = gf_evidence_workspace("gf_scan_evidence_sources", (size_t)nscales * nsrc, nx, p.ny, d_work, work_bytes, st, &part, &tickets))
+        return rc;
+    kern<<<dim3(nx, (unsigned)p.ny), GF_EVS_THREADS, smem, st>>>(d, tab, cfg->seed, cfg->first_index, cfg->count, d_scales, nscales, p.s_per, p.G,
+                                                                 p.slots, part, tickets, d_lse);
     ++g_gf_launches;
     GF_LAUNCH_CHECK("gf_scan_evidence_sources");
     return GF_OK;

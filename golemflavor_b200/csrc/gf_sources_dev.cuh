@@ -41,6 +41,10 @@ GF_HD bool gf_src_record(const double* s, const double* inj, double W, gf_src_re
     return true;
 }
 
+/* The source table of a source-list entry point `who` (host): refuses a model that samples the source or has no Gaussian
+ * likelihood, and a composition gf_src_record refuses; fills S from sources[nsrc][3] / injected[nsrc][3] otherwise. */
+int gf_src_table_fill(const char* who, const gf_dev_model& d, const double* sources, const double* injected, int nsrc, gf_src_table* S);
+
 /* llh.multi_gaussian of source r's composition fr (written) from the transition sums A of one (sample, scale) */
 GF_HD double gf_src_llh(const gf_dev_model& m, const gf_src_rec& r, const double* A, double* fr) {
     gfp_transition_fr(A, r.c, fr);
@@ -52,32 +56,8 @@ GF_HD double gf_src_llh(const gf_dev_model& m, const gf_src_rec& r, const double
     return gf_src_llh(m, r, A, fr);
 }
 
-/* running log-sum-exp (max, sum) += one likelihood: the update rule of k_evidence_grid.  NaN and -inf (pdf underflow)
- * carry no weight. */
-GF_HD void gf_src_lse_push(double& mo, double& so, double ll) {
-    if (ll > -INFINITY) {
-        const double d = ll - mo; /* +inf on the first sample */
-        const double e = exp(-fabs(d));
-        if (d <= 0.0) {
-            so += e;
-        } else {
-            so = fma(so, e, 1.0);
-            mo = ll;
-        }
-    }
-}
-
-/* (m, s) <- log-sum-exp merge of two partials; empty partials are (-inf, 0) (gf_lse_merge of gf_scan.cu) */
-GF_HD void gf_src_lse_merge(double& m, double& s, double m2, double s2) {
-    const double mm = fmax(m, m2);
-    if (mm == -INFINITY) {
-        m = -INFINITY;
-        s = 0.0;
-        return;
-    }
-    s = s * exp(m - mm) + s2 * exp(m2 - mm);
-    m = mm;
-}
+/* the running log-sum-exp of one (scale, source) pair: gf_lse_push, under the name the source grid's host harness calls */
+GF_HD void gf_src_lse_push(double& mo, double& so, double ll) { gf_lse_push(mo, so, ll); }
 
 /* The physics of prior sample `index` (the draw of gf_scan_evidence_grid) at the ns scales lam[0..ns-1]:
  * emit(k, A, status) per scale.  STATIC6: the layout of sens.py, columns 0-3 mixing coordinates, 4-5 mass splittings. */

@@ -240,13 +240,8 @@ def scan_evidence(fm, count, seed=26, first_index=0, distributed=True):
     cfg = _lib.ScanConfig(seed=int(seed), first_index=int(start), count=int(n), nb=0)
     _lib.check(_lib.load().gf_scan_evidence(fm.ref, C.byref(cfg), _lib.ptr(lse), _lib.stream_ptr(torch)))
     if dist and world > 1:
-        gmax = lse[:1].clone()
-        dist.all_reduce(gmax, op=dist.ReduceOp.MAX)
-        part = lse[1:] * torch.exp(lse[:1] - gmax) if bool(torch.isfinite(gmax)) else lse[1:] * 0
-        dist.all_reduce(part, op=dist.ReduceOp.SUM)
-        lse = torch.cat([gmax, part])
-    m, s = (float(x) for x in lse.cpu())
-    return m + np.log(s) - np.log(count) if s > 0 else -np.inf
+        lse = _lse_allreduce(dist, lse)
+    return float(_lnz(lse.cpu().numpy(), count))
 
 
 def scan_evidence_grid(fm, scales, count, seed=26, first_index=0, distributed=True):
@@ -268,14 +263,8 @@ def scan_evidence_grid(fm, scales, count, seed=26, first_index=0, distributed=Tr
     cfg = _lib.ScanConfig(seed=int(seed), first_index=int(start), count=int(n), nb=0)
     _lib.check(lib.gf_scan_evidence_grid(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, _lib.ptr(lse), _lib.ptr(work), nbytes, _lib.stream_ptr(torch)))
     if dist and world > 1:
-        gmax = lse[:, 0].clone()
-        dist.all_reduce(gmax, op=dist.ReduceOp.MAX)
-        part = torch.where(torch.isfinite(gmax), lse[:, 1] * torch.exp(lse[:, 0] - gmax), torch.zeros_like(gmax))
-        dist.all_reduce(part, op=dist.ReduceOp.SUM)
-        lse = torch.stack([gmax, part], dim=1)
-    h = lse.cpu().numpy()
-    with np.errstate(divide='ignore'):
-        return np.where(h[:, 1] > 0, h[:, 0] + np.log(h[:, 1]) - np.log(count), -np.inf)
+        lse = _lse_allreduce(dist, lse)
+    return _lnz(lse.cpu().numpy(), count)
 
 
 def source_rows(sources, injected):
@@ -306,22 +295,22 @@ def _sources_launch(lib, fm, cfg, sc, ns, src, inj, lse, stream):
         s, i = src[j0:j0 + _lib.GF_SRC_MAX], inj[j0:j0 + _lib.GF_SRC_MAX]
         n = s.shape[0]
         nbytes = int(lib.gf_scan_evidence_sources_workspace(ns, n))
-        work = _sources_workspace(torch, nbytes)
+        work = _workspace(torch, nbytes)
         _lib.check(lib.gf_scan_evidence_sources(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, s.ctypes.data_as(C.c_void_p),
                                                 i.ctypes.data_as(C.c_void_p), n, C.c_void_p(lse.data_ptr() + 16 * ns * j0),
                                                 _lib.ptr(work), nbytes, stream))
 
 
-_SRC_WORK = {}
+_WORK = {}
 
 
-def _sources_workspace(torch, nbytes):
-    """Scratch of the source-grid kernel, one buffer per (device, stream), grown on demand and reused by later calls (the
-    kernel leaves it reusable by the next launch on the same stream)."""
+def _workspace(torch, nbytes):
+    """Scratch of the evidence-grid kernels, one buffer per (device, stream), grown on demand and reused by later calls (the
+    kernels leave it reusable by the next launch on the same stream)."""
     key = (torch.cuda.current_device(), torch.cuda.current_stream().cuda_stream)
-    buf = _SRC_WORK.get(key)
+    buf = _WORK.get(key)
     if buf is None or buf.numel() < nbytes:
-        buf = _SRC_WORK[key] = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device='cuda')
+        buf = _WORK[key] = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device='cuda')
     return buf
 
 
@@ -336,6 +325,7 @@ def _lse_allreduce(dist, lse):
 
 
 def _lnz(h, count):
+    """ln( (1/count) sum ) of (max, sum-exp) pairs [..., 2]; -inf where no sample carried weight."""
     with np.errstate(divide='ignore'):
         return np.where(h[..., 1] > 0, h[..., 0] + np.log(h[..., 1]) - np.log(count), -np.inf)
 
@@ -387,20 +377,25 @@ def scan_profile_grid(fm, scales, nstarts=PROFILE_NSTARTS, seed=27, task0=0, max
                 nconverged=c[:, 1])
 
 
-def _profile_launch(torch, fm, scales, nstarts, seed, task0, max_evals=PROFILE_MAX_EVALS, ftol=PROFILE_FTOL, xtol=PROFILE_XTOL):
-    """Enqueue ``gf_profile_grid`` on torch's current stream: (best, argmax, fr, status, counts) as CUDA tensors."""
+def _profile_setup(torch, fm, scales, lead, nstarts, seed, task0, max_evals, ftol, xtol):
+    """(scales on the device, their number, ProfileConfig, outputs) of a profile launch; the outputs (best, argmax, fr, status,
+    counts) are CUDA tensors with the leading axes ``lead`` before the scale axis."""
     sc = torch.as_tensor(np.ascontiguousarray(scales, dtype=np.float64).ravel()).cuda()
     ns = int(sc.numel())
-    best = torch.empty((ns,), dtype=torch.float64, device='cuda')
-    argmax = torch.empty((ns, fm.ndim), dtype=torch.float64, device='cuda')
-    fr = torch.empty((ns, 3), dtype=torch.float64, device='cuda')
-    st = torch.empty((ns,), dtype=torch.uint8, device='cuda')
-    counts = torch.empty((ns, 2), dtype=torch.int64, device='cuda')
+    shape = tuple(lead) + (ns,)
+    out = (torch.empty(shape, dtype=torch.float64, device='cuda'), torch.empty(shape + (fm.ndim,), dtype=torch.float64, device='cuda'),
+           torch.empty(shape + (3,), dtype=torch.float64, device='cuda'), torch.empty(shape, dtype=torch.uint8, device='cuda'),
+           torch.empty(shape + (2,), dtype=torch.int64, device='cuda'))
     cfg = _lib.ProfileConfig(seed=int(seed), task0=int(task0), nstarts=int(nstarts), max_evals=int(max_evals), ftol=float(ftol),
                              xtol=float(xtol))
-    _lib.check(_lib.load().gf_profile_grid(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, _lib.ptr(best), _lib.ptr(argmax), _lib.ptr(fr),
-                                           _lib.ptr(st), _lib.ptr(counts), _lib.stream_ptr(torch)))
-    return best, argmax, fr, st, counts
+    return sc, ns, cfg, out
+
+
+def _profile_launch(torch, fm, scales, nstarts, seed, task0, max_evals=PROFILE_MAX_EVALS, ftol=PROFILE_FTOL, xtol=PROFILE_XTOL):
+    """Enqueue ``gf_profile_grid`` on torch's current stream: (best, argmax, fr, status, counts) as CUDA tensors."""
+    sc, ns, cfg, out = _profile_setup(torch, fm, scales, (), nstarts, seed, task0, max_evals, ftol, xtol)
+    _lib.check(_lib.load().gf_profile_grid(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, *(_lib.ptr(t) for t in out), _lib.stream_ptr(torch)))
+    return out
 
 
 def scan_profile_sources(fm, scales, sources, injected, nstarts=PROFILE_NSTARTS, seed=27, task0=0, max_evals=PROFILE_MAX_EVALS, ftol=PROFILE_FTOL,
@@ -420,19 +415,10 @@ def scan_profile_sources(fm, scales, sources, injected, nstarts=PROFILE_NSTARTS,
 def _profile_sources_launch(torch, fm, scales, src, inj, nstarts, seed, task0, max_evals=PROFILE_MAX_EVALS, ftol=PROFILE_FTOL, xtol=PROFILE_XTOL):
     """Enqueue ``gf_profile_sources`` on torch's current stream for the validated rows ``src`` / ``inj`` (any number: split into
     calls of at most ``GF_SRC_MAX``): (best, argmax, fr, status, counts) as CUDA tensors with a leading [nsrc] axis."""
-    sc = torch.as_tensor(np.ascontiguousarray(scales, dtype=np.float64).ravel()).cuda()
-    ns, nsrc = int(sc.numel()), src.shape[0]
-    best = torch.empty((nsrc, ns), dtype=torch.float64, device='cuda')
-    argmax = torch.empty((nsrc, ns, fm.ndim), dtype=torch.float64, device='cuda')
-    fr = torch.empty((nsrc, ns, 3), dtype=torch.float64, device='cuda')
-    st = torch.empty((nsrc, ns), dtype=torch.uint8, device='cuda')
-    counts = torch.empty((nsrc, ns, 2), dtype=torch.int64, device='cuda')
-    cfg = _lib.ProfileConfig(seed=int(seed), task0=int(task0), nstarts=int(nstarts), max_evals=int(max_evals), ftol=float(ftol),
-                             xtol=float(xtol))
+    sc, ns, cfg, out = _profile_setup(torch, fm, scales, (src.shape[0],), nstarts, seed, task0, max_evals, ftol, xtol)
     lib, stream = _lib.load(), _lib.stream_ptr(torch)
-    for j0 in range(0, nsrc, _lib.GF_SRC_MAX):
+    for j0 in range(0, src.shape[0], _lib.GF_SRC_MAX):
         s, i = src[j0:j0 + _lib.GF_SRC_MAX], inj[j0:j0 + _lib.GF_SRC_MAX]
         _lib.check(lib.gf_profile_sources(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, s.ctypes.data_as(C.c_void_p), i.ctypes.data_as(C.c_void_p),
-                                          s.shape[0], _lib.ptr(best[j0]), _lib.ptr(argmax[j0]), _lib.ptr(fr[j0]), _lib.ptr(st[j0]),
-                                          _lib.ptr(counts[j0]), stream))
-    return best, argmax, fr, st, counts
+                                          s.shape[0], *(_lib.ptr(t[j0]) for t in out), stream))
+    return out

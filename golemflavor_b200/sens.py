@@ -20,7 +20,7 @@ from .enums import ParamTag, Texture
 from .mcmc import DeviceEnsembleSampler
 from .param import Param, ParamSet
 from .scan import (DEFAULT_BINNING, PROFILE_NSTARTS, _dist, _lnz, _lse_allreduce, _profile_launch, _profile_sources_launch, _sources_launch,
-                   shard_range, sm_paramset, source_rows)
+                   _workspace, shard_range, sm_paramset, source_rows)
 
 __all__ = ['scale_grid', 'sweep_paramset', 'sweep', 'evidence_grid', 'evidence_source_grid', 'profile_grid', 'profile_source_grid', 'get_limit',
            'limits', 'limit_table', 'BAYES_K', 'FREQ_CL']
@@ -165,20 +165,13 @@ def evidence_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.O
     work_bytes = int(lib.gf_scan_evidence_grid_workspace(max(nsc)))
     work = _workspace(torch, work_bytes)
     for k, dim in enumerate(dims):
-        args = Namespace(source_ratio=src / src.sum(), dimension=dim, texture=texture, binning=np.asarray(binning),
-                         no_bsm=False, injected_ratio=inj / inj.sum(), smearing=float(smearing), fixed_scale=-100.0)
-        fm = _model.flatten(args, None, ParamSet(sm_paramset(with_mass=True)))
+        fm = _grid_model(dim, texture, src, inj, smearing, binning)
         _lib.check(lib.gf_scan_evidence_grid(fm.ref, C.byref(cfg), C.c_void_p(scales.data_ptr() + 8 * int(offs[k])), nsc[k],
                                              C.c_void_p(lse.data_ptr() + 16 * int(offs[k])), _lib.ptr(work), work_bytes, stream))
     if dist and world > 1:
-        gmax = lse[:, 0].clone()
-        dist.all_reduce(gmax, op=dist.ReduceOp.MAX)
-        part = torch.where(torch.isfinite(gmax), lse[:, 1] * torch.exp(lse[:, 0] - gmax), torch.zeros_like(gmax))
-        dist.all_reduce(part, op=dist.ReduceOp.SUM)
-        lse = torch.stack([gmax, part], dim=1)
+        lse = _lse_allreduce(dist, lse)
     h = lse.cpu().numpy()
-    with np.errstate(divide='ignore'):
-        lnz = np.where(h[:, 1] > 0, h[:, 0] + np.log(h[:, 1]) - np.log(samples), -np.inf)
+    lnz = _lnz(h, samples)
     allsc = np.concatenate(grids)
     ev = {d: np.column_stack([allsc[offs[k]:offs[k + 1]], lnz[offs[k]:offs[k + 1]]]) for k, d in enumerate(dims)}
     if return_maxllh:
@@ -187,8 +180,8 @@ def evidence_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.O
 
 
 def _grid_model(dim, texture, src, inj, smearing, binning):
-    """The six SM nuisance parameters with the scale frozen (``sens.py:261-266``), built exactly as ``evidence_grid`` builds
-    its model; the kernel substitutes each grid scale."""
+    """The six SM nuisance parameters with the scale frozen (``sens.py:261-266``), the model of every sensitivity grid; the
+    kernels substitute each grid scale."""
     args = Namespace(source_ratio=src / src.sum(), dimension=int(dim), texture=texture, binning=np.asarray(binning),
                      no_bsm=False, injected_ratio=inj / inj.sum(), smearing=float(smearing), fixed_scale=-100.0)
     return _model.flatten(args, None, ParamSet(sm_paramset(with_mass=True)))
@@ -245,37 +238,17 @@ def profile_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OE
     The grid points are sharded over the ranks of the process group (``task0`` = index of the scale in its dimension's grid)
     and the disjoint rows are merged with one all-reduce: the result is the same for any number of ranks."""
     torch = _lib.torch_cuda()
-    dist = _dist() if distributed else None
-    rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
     src = np.asarray(source_ratio, dtype=np.float64)
     inj = np.asarray(injected_ratio, dtype=np.float64)
     dims = [int(d) for d in dimensions]
     segments = int(segments)
-    grid = [(k, s) for k in range(len(dims)) for s in range(segments)]
-    start, count = shard_range(len(grid), rank, world)
-    ndim = len(sm_paramset(with_mass=True))
-    rows = np.zeros((len(grid), 1 + ndim))
-    cur = torch.cuda.current_stream()
-    pending = []
-    for k, dim in enumerate(dims):
-        mine = [s for kk, s in grid[start:start + count] if kk == k]
-        if not mine:
-            continue
+
+    def launch(dim, scales, task0):
         fm = _grid_model(dim, texture, src, inj, smearing, binning)
-        scales = scale_grid(dim, segments)[mine[0]:mine[-1] + 1]
-        stream = _dim_stream(torch, dim)
-        stream.wait_stream(cur)
-        with torch.cuda.stream(stream):
-            out = _profile_launch(torch, fm, scales, nstarts, seed, mine[0])
-        pending.append((stream, k * segments + mine[0], out))
-    for stream, row0, (best, argmax, _, _, _) in pending:
-        stream.synchronize()
-        rows[row0:row0 + best.numel(), 0] = best.cpu().numpy()
-        rows[row0:row0 + best.numel(), 1:] = argmax.cpu().numpy()
-    if dist and world > 1:
-        t = torch.as_tensor(rows).cuda()
-        dist.all_reduce(t, op=dist.ReduceOp.SUM)                   # disjoint rows: sum == gather
-        rows = t.cpu().numpy()
+        best, argmax = _profile_launch(torch, fm, scales, nstarts, seed, task0)[:2]
+        return best[None], argmax[None]
+
+    rows = _profile_rows(dims, segments, 1, distributed, launch)[:, 0]
     prof = {d: np.column_stack([scale_grid(d, segments), rows[k * segments:(k + 1) * segments, 0]]) for k, d in enumerate(dims)}
     if return_argmax:
         return prof, {d: rows[k * segments:(k + 1) * segments, 1:].copy() for k, d in enumerate(dims)}
@@ -298,38 +271,15 @@ def profile_source_grid(sources, dimensions=(3, 4, 5, 6, 7, 8), segments=100, te
     the result is the same for any number of ranks."""
     src, inj = source_rows(sources, injected_ratio)
     torch = _lib.torch_cuda()
-    dist = _dist() if distributed else None
-    rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
     dims = [int(d) for d in dimensions]
     segments = int(segments)
-    nsrc = src.shape[0]
-    grid = [(k, s) for k in range(len(dims)) for s in range(segments)]
-    start, count = shard_range(len(grid), rank, world)
-    ndim = len(sm_paramset(with_mass=True))
-    rows = np.zeros((len(grid), nsrc, 1 + ndim))
-    cur = torch.cuda.current_stream()
-    pending = []
-    # the model's own source and injected composition are ignored by the kernel: the first row stands in
-    for k, dim in enumerate(dims):
-        mine = [s for kk, s in grid[start:start + count] if kk == k]
-        if not mine:
-            continue
+
+    def launch(dim, scales, task0):
+        # the model's own source and injected composition are ignored by the kernel: the first row stands in
         fm = _grid_model(dim, texture, src[0], inj[0], smearing, binning)
-        scales = scale_grid(dim, segments)[mine[0]:mine[-1] + 1]
-        stream = _dim_stream(torch, dim)
-        stream.wait_stream(cur)
-        with torch.cuda.stream(stream):
-            out = _profile_sources_launch(torch, fm, scales, src, inj, nstarts, seed, mine[0])
-        pending.append((stream, k * segments + mine[0], out))
-    for stream, row0, (best, argmax, _, _, _) in pending:
-        stream.synchronize()
-        n = best.shape[1]
-        rows[row0:row0 + n, :, 0] = best.cpu().numpy().T
-        rows[row0:row0 + n, :, 1:] = argmax.cpu().numpy().transpose(1, 0, 2)
-    if dist and world > 1:
-        t = torch.as_tensor(rows).cuda()
-        dist.all_reduce(t, op=dist.ReduceOp.SUM)                   # disjoint rows: sum == gather
-        rows = t.cpu().numpy()
+        return _profile_sources_launch(torch, fm, scales, src, inj, nstarts, seed, task0)[:2]
+
+    rows = _profile_rows(dims, segments, src.shape[0], distributed, launch)
     prof = {}
     for k, d in enumerate(dims):
         r = rows[k * segments:(k + 1) * segments].transpose(1, 0, 2)          # [nsrc, segments, 1 + ndim]
@@ -339,16 +289,39 @@ def profile_source_grid(sources, dimensions=(3, 4, 5, 6, 7, 8), segments=100, te
     return prof
 
 
-_WORK = {}
-
-
-def _workspace(torch, nbytes):
-    """Scratch of the grid kernel, allocated once per (device, size class) and reused by later calls."""
-    key = torch.cuda.current_device()
-    buf = _WORK.get(key)
-    if buf is None or buf.numel() < nbytes:
-        buf = _WORK[key] = torch.empty(int(nbytes), dtype=torch.uint8, device='cuda')
-    return buf
+def _profile_rows(dims, segments, nsrc, distributed, launch):
+    """The rows [len(dims) * segments, nsrc, 1 + 6] of (profile, argmax) of a profile grid.  The (dimension, scale) rows are
+    sharded over the ranks of the process group; this rank's rows of a dimension run as ``launch(dim, scales, task0)`` -> (best
+    [nsrc, n], argmax [nsrc, n, 6]) CUDA tensors on the dimension's stream, ``task0`` the index of ``scales[0]`` in the
+    dimension's grid.  The disjoint rows of the ranks are merged with one all-reduce."""
+    torch = _lib.torch_cuda()
+    dist = _dist() if distributed else None
+    rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
+    grid = [(k, s) for k in range(len(dims)) for s in range(segments)]
+    start, count = shard_range(len(grid), rank, world)
+    ndim = len(sm_paramset(with_mass=True))
+    rows = np.zeros((len(grid), nsrc, 1 + ndim))
+    cur = torch.cuda.current_stream()
+    pending = []
+    for k, dim in enumerate(dims):
+        mine = [s for kk, s in grid[start:start + count] if kk == k]
+        if not mine:
+            continue
+        stream = _dim_stream(torch, dim)
+        stream.wait_stream(cur)
+        with torch.cuda.stream(stream):
+            out = launch(dim, scale_grid(dim, segments)[mine[0]:mine[-1] + 1], mine[0])
+        pending.append((stream, k * segments + mine[0], out))
+    for stream, row0, (best, argmax) in pending:
+        stream.synchronize()
+        n = best.shape[1]
+        rows[row0:row0 + n, :, 0] = best.cpu().numpy().T
+        rows[row0:row0 + n, :, 1:] = argmax.cpu().numpy().transpose(1, 0, 2)
+    if dist and world > 1:
+        t = torch.as_tensor(rows).cuda()
+        dist.all_reduce(t, op=dist.ReduceOp.SUM)                   # disjoint rows: sum == gather
+        rows = t.cpu().numpy()
+    return rows
 
 
 BAYES_K = 1.   # golemflavor/plot.py:82: "Strong degree of belief"
