@@ -56,4 +56,9 @@ unsigned gf_evidence_nx(int sms, int per_sm, int ny, uint64_t count, int threads
 int gf_evidence_workspace(const char* who, size_t rows, unsigned nx, int ny, void* d_work, uint64_t work_bytes, cudaStream_t st, double** part,
                           unsigned int** tickets);
 
+/* Sample groups of the grouped evidence grids (sample i in group i mod groups): a power of two in [2, 32], so that a group
+ * is fixed per thread of the grid kernel and per lane of a warp. */
+#define GF_EVIDENCE_MAX_GROUPS 32
+bool gf_evidence_groups_ok(int groups);
+
 #endif /* GF_COMMON_CUH */

@@ -670,23 +670,31 @@ extern "C" int gf_scan_evidence(const gf_model* model, const gf_scan_config* cfg
  * every (thread, scale) lives in shared memory (two LDS/STS per ~1900 fp64 instructions), so the accumulators cost no
  * registers.  Per-block partials are merged by the LAST block of the group (ticket counter) in block order:
  * deterministic for a given launch geometry, no finishing kernel, no allocation.
+ *
+ * GROUPED: the samples are split into R = `groups` fixed groups (R a power of two dividing 32), sample i in group i mod R,
+ * and every (scale, group) gets its own (max, sum) -- the input of a delete-one-group jackknife of lnZ.  The sample stride is
+ * a multiple of T and R divides T, so a thread's samples all lie in group (first_index + tid) mod R: the physics loop is
+ * untouched, the block reduction merges lanes by shuffle down to offset R (lane l < R then holds residue class l of its
+ * warp) and warps in order, and the partials are [nscales][R][gridDim.x][2].  Without GROUPED R is 1 and the kernel is the
+ * ungrouped one; `groups` is never read.
  */
 #define GF_EVG_MAX_S_PER 16
 
-template <int SPEC, bool STATIC6>
+template <int SPEC, bool STATIC6, bool GROUPED = false>
 __global__ void __launch_bounds__(GF_SCAN_THREADS, GF_SCAN_MIN_BLOCKS)
     k_evidence_grid(const __grid_constant__ gf_dev_model m, const uint64_t seed, const uint64_t first_index, const uint64_t count,
-                    const double* __restrict__ scales, const int nscales, const int s_per, double* __restrict__ partials /*[nscales][gridDim.x][2]*/,
-                    unsigned int* __restrict__ tickets /*[gridDim.y]*/, double* __restrict__ lse /*[nscales][2]*/) {
+                    const double* __restrict__ scales, const int nscales, const int s_per, double* __restrict__ partials /*[nscales][R][gridDim.x][2]*/,
+                    unsigned int* __restrict__ tickets /*[gridDim.y]*/, double* __restrict__ lse /*[nscales][R][2]*/, const int groups) {
     extern __shared__ double sh_evg[];
     constexpr int T = GF_SCAN_THREADS, W = GF_SCAN_THREADS / 32;
     double* sh_lam = sh_evg;                        /* [GF_EVG_MAX_S_PER]        */
     double* sh_m = sh_evg + GF_EVG_MAX_S_PER;       /* [s_per][T] running max    */
     double* sh_s = sh_m + s_per * T;                /* [s_per][T] running sum    */
-    __shared__ double sh_wm[GF_EVG_MAX_S_PER][W], sh_ws[GF_EVG_MAX_S_PER][W];
+    __shared__ double sh_wm[GROUPED ? 1 : GF_EVG_MAX_S_PER][W], sh_ws[GROUPED ? 1 : GF_EVG_MAX_S_PER][W];
     __shared__ int sh_last;
     const int tid = threadIdx.x, g = blockIdx.y;
     const int s0 = g * s_per, ns = min(s_per, nscales - s0);
+    const int R = GROUPED ? groups : 1;
     if (tid < ns) sh_lam[tid] = exp10(scales[s0 + tid]); /* the same exp10 the per-point kernels apply to logLam */
     for (int k = 0; k < ns; ++k) {
         sh_m[k * T + tid] = -INFINITY;
@@ -719,24 +727,33 @@ __global__ void __launch_bounds__(GF_SCAN_THREADS, GF_SCAN_MIN_BLOCKS)
                 }
             });
     }
-    /* block reduction: lanes by shuffle, warps in order */
+    /* block reduction: lanes by shuffle (down to offset R), warps in order */
     const int lane = tid & 31, warp = tid >> 5;
     for (int k = 0; k < ns; ++k) {
         double mx = sh_m[k * T + tid], sm = sh_s[k * T + tid];
-        for (int o = 16; o > 0; o >>= 1) {
+        for (int o = 16; o >= R; o >>= 1) {
             const double m2 = __shfl_down_sync(0xffffffffu, mx, o), s2 = __shfl_down_sync(0xffffffffu, sm, o);
             gf_lse_merge(mx, sm, m2, s2);
         }
-        if (lane == 0) {
-            sh_wm[k][warp] = mx;
-            sh_ws[k][warp] = sm;
+        if (lane < R) {
+            if constexpr (GROUPED) { /* each thread overwrites only its own accumulator, which only it has read */
+                sh_m[k * T + tid] = mx;
+                sh_s[k * T + tid] = sm;
+            } else {
+                sh_wm[k][warp] = mx;
+                sh_ws[k][warp] = sm;
+            }
         }
     }
     __syncthreads();
-    if (tid < ns) {
-        double mx = sh_wm[tid][0], sm = sh_ws[tid][0];
-        for (int w = 1; w < W; ++w) gf_lse_merge(mx, sm, sh_wm[tid][w], sh_ws[tid][w]);
-        double* out = partials + 2 * ((size_t)(s0 + tid) * gridDim.x + blockIdx.x);
+    /* one thread per (scale, group): k = tid / R, group r = (first_index + lane) mod R holds lane l of every warp */
+    const int kk = tid / R, r = tid - kk * R, l = (r - (int)(first_index & (uint64_t)(R - 1))) & (R - 1);
+    if (tid < ns * R) {
+        auto wm = [&](int w) { if constexpr (GROUPED) return sh_m[kk * T + 32 * w + l]; else return sh_wm[kk][w]; };
+        auto ws = [&](int w) { if constexpr (GROUPED) return sh_s[kk * T + 32 * w + l]; else return sh_ws[kk][w]; };
+        double mx = wm(0), sm = ws(0);
+        for (int w = 1; w < W; ++w) gf_lse_merge(mx, sm, wm(w), ws(w));
+        double* out = partials + 2 * (((size_t)(s0 + kk) * R + r) * gridDim.x + blockIdx.x);
         out[0] = mx;
         out[1] = sm;
     }
@@ -747,12 +764,13 @@ __global__ void __launch_bounds__(GF_SCAN_THREADS, GF_SCAN_MIN_BLOCKS)
     __syncthreads();
     if (!sh_last) return;
     __threadfence();
-    if (tid < ns) {
-        double mx = lse[2 * (s0 + tid)], sm = lse[2 * (s0 + tid) + 1];
-        const volatile double* in = partials + 2 * (size_t)(s0 + tid) * gridDim.x;
+    if (tid < ns * R) {
+        const int row = (s0 + kk) * R + r;
+        double mx = lse[2 * row], sm = lse[2 * row + 1];
+        const volatile double* in = partials + 2 * (size_t)row * gridDim.x;
         for (unsigned b = 0; b < gridDim.x; ++b) gf_lse_merge(mx, sm, in[2 * b], in[2 * b + 1]); /* block order: deterministic */
-        lse[2 * (s0 + tid)] = mx;
-        lse[2 * (s0 + tid) + 1] = sm;
+        lse[2 * row] = mx;
+        lse[2 * row + 1] = sm;
     }
     if (tid == 0) tickets[g] = 0u; /* the workspace is reusable by the next launch on this stream */
 }
@@ -766,12 +784,14 @@ struct evg_geometry {
 };
 
 template <class K>
-int evg_plan(K kern, int nscales, uint64_t count, evg_geometry* geo) {
+int evg_plan(K kern, int nscales, uint64_t count, int groups, evg_geometry* geo) {
     int sms = 0;
     if (int rc = gf_sm_count(&sms)) return rc;
     /* scales per block: as many as amortise the per-sample set-up while every SM still gets work; 10 scales
-     * (20 KB of accumulators per block... 2 x 10 x 256 x 8 B = 40 KB) leave two blocks per SM */
+     * (20 KB of accumulators per block... 2 x 10 x 256 x 8 B = 40 KB) leave two blocks per SM.  With groups, one thread
+     * per (scale, group) merges the block's partials: s_per * groups <= T (8 scales at 32 groups) */
     int s_per = nscales < 10 ? nscales : 10;
+    if (s_per * groups > GF_SCAN_THREADS) s_per = GF_SCAN_THREADS / groups;
     const size_t smem = (size_t)(GF_EVG_MAX_S_PER + 2 * s_per * GF_SCAN_THREADS) * sizeof(double);
     GF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 1;
@@ -810,32 +830,65 @@ int gf_evidence_workspace(const char* who, size_t rows, unsigned nx, int ny, voi
     return GF_OK;
 }
 
-extern "C" uint64_t gf_scan_evidence_grid_workspace(int32_t nscales) {
+namespace {
+
+/* [nscales][groups][blocks in x][2] partials (blocks in x <= resident blocks of the device) + one ticket per scale; 0 if refused */
+uint64_t evidence_grid_workspace(int32_t nscales, int groups) {
     int sms = 0;
     if (nscales < 1 || gf_sm_count(&sms) != GF_OK) return 0;
-    /* [nscales][blocks in x][2] partials (blocks in x <= resident blocks of the device) + one ticket per scale */
-    return (uint64_t)nscales * ((uint64_t)sms * 8) * 2 * sizeof(double) + (uint64_t)nscales * sizeof(unsigned int) + 256;
+    return (uint64_t)nscales * groups * ((uint64_t)sms * 8) * 2 * sizeof(double) + (uint64_t)nscales * sizeof(unsigned int) + 256;
 }
+
+}  // namespace
+
+extern "C" uint64_t gf_scan_evidence_grid_workspace(int32_t nscales) { return evidence_grid_workspace(nscales, 1); }
+
+extern "C" uint64_t gf_scan_evidence_grid_groups_workspace(int32_t nscales, int32_t groups) {
+    return gf_evidence_groups_ok(groups) ? evidence_grid_workspace(nscales, groups) : 0;
+}
+
+bool gf_evidence_groups_ok(int groups) { return groups >= 2 && groups <= GF_EVIDENCE_MAX_GROUPS && (groups & (groups - 1)) == 0; }
+
+namespace {
+
+/* gf_scan_evidence_grid (grouped = false: the ungrouped kernel, lse [nscales][2]) and gf_scan_evidence_grid_groups (lse
+ * [nscales][groups][2]): the same checks, plan and launch */
+int evidence_grid(const char* who, const gf_model* model, const gf_scan_config* cfg, const double* d_scales, int32_t nscales, bool grouped,
+                  int groups, double* d_lse, void* d_work, uint64_t work_bytes, cudaStream_t st) {
+    GF_REQUIRE(cfg != nullptr && d_lse != nullptr && d_scales != nullptr, "%s: null pointer", who);
+    GF_REQUIRE(nscales >= 1 && nscales <= 65535, "%s: nscales = %d outside [1, 65535]", who, nscales);
+    GF_REQUIRE(!grouped || gf_evidence_groups_ok(groups), "%s: groups = %d is not a power of two in [2, %d]", who, groups,
+               GF_EVIDENCE_MAX_GROUPS);
+    gf_dev_model d;
+    if (int rc = gf_build_dev_model(model, &d)) return rc;
+    if (int rc = gf_check_frozen_scale(who, d)) return rc;
+    if (cfg->count == 0) return GF_OK;
+    const int spec = gf_model_grid_spec(d);
+    auto kern = grouped ? (spec == 2 ? k_evidence_grid<GF_SPEC_FIXED, true, true> : spec == 1 ? k_evidence_grid<GF_SPEC_FIXED, false, true>
+                                                                                              : k_evidence_grid<GF_SPEC_GENERIC, false, true>)
+                       : (spec == 2 ? k_evidence_grid<GF_SPEC_FIXED, true> : spec == 1 ? k_evidence_grid<GF_SPEC_FIXED, false>
+                                                                                       : k_evidence_grid<GF_SPEC_GENERIC, false>);
+    const int R = grouped ? groups : 1;
+    evg_geometry geo;
+    if (int rc = evg_plan(kern, nscales, cfg->count, R, &geo)) return rc;
+    double* part = nullptr;
+    unsigned int* tickets = nullptr;
+    if (int rc = gf_evidence_workspace(who, (size_t)nscales * R, geo.nx, geo.ny, d_work, work_bytes, st, &part, &tickets)) return rc;
+    kern<<<dim3(geo.nx, (unsigned)geo.ny), GF_SCAN_THREADS, geo.smem, st>>>(d, cfg->seed, cfg->first_index, cfg->count, d_scales, nscales, geo.s_per, part,
+                                                                              tickets, d_lse, R);
+    ++g_gf_launches;
+    GF_LAUNCH_CHECK(who);
+    return GF_OK;
+}
+
+}  // namespace
 
 extern "C" int gf_scan_evidence_grid(const gf_model* model, const gf_scan_config* cfg, const double* d_scales, int32_t nscales,
                                      double* d_lse, void* d_work, uint64_t work_bytes, void* stream) {
-    GF_REQUIRE(cfg != nullptr && d_lse != nullptr && d_scales != nullptr, "gf_scan_evidence_grid: null pointer");
-    GF_REQUIRE(nscales >= 1 && nscales <= 65535, "gf_scan_evidence_grid: nscales = %d outside [1, 65535]", nscales);
-    gf_dev_model d;
-    if (int rc = gf_build_dev_model(model, &d)) return rc;
-    if (int rc = gf_check_frozen_scale("gf_scan_evidence_grid", d)) return rc;
-    if (cfg->count == 0) return GF_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int spec = gf_model_grid_spec(d);
-    auto kern = spec == 2 ? k_evidence_grid<GF_SPEC_FIXED, true> : spec == 1 ? k_evidence_grid<GF_SPEC_FIXED, false> : k_evidence_grid<GF_SPEC_GENERIC, false>;
-    evg_geometry geo;
-    if (int rc = evg_plan(kern, nscales, cfg->count, &geo)) return rc;
-    double* part = nullptr;
-    unsigned int* tickets = nullptr;
-    if (int rc = gf_evidence_workspace("gf_scan_evidence_grid", nscales, geo.nx, geo.ny, d_work, work_bytes, st, &part, &tickets)) return rc;
-    kern<<<dim3(geo.nx, (unsigned)geo.ny), GF_SCAN_THREADS, geo.smem, st>>>(d, cfg->seed, cfg->first_index, cfg->count, d_scales, nscales, geo.s_per, part,
-                                                                              tickets, d_lse);
-    ++g_gf_launches;
-    GF_LAUNCH_CHECK("gf_scan_evidence_grid");
-    return GF_OK;
+    return evidence_grid("gf_scan_evidence_grid", model, cfg, d_scales, nscales, false, 1, d_lse, d_work, work_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int gf_scan_evidence_grid_groups(const gf_model* model, const gf_scan_config* cfg, const double* d_scales, int32_t nscales,
+                                            int32_t groups, double* d_lse, void* d_work, uint64_t work_bytes, void* stream) {
+    return evidence_grid("gf_scan_evidence_grid_groups", model, cfg, d_scales, nscales, true, groups, d_lse, d_work, work_bytes, (cudaStream_t)stream);
 }

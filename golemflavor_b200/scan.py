@@ -244,27 +244,91 @@ def scan_evidence(fm, count, seed=26, first_index=0, distributed=True):
     return float(_lnz(lse.cpu().numpy(), count))
 
 
-def scan_evidence_grid(fm, scales, count, seed=26, first_index=0, distributed=True):
+def scan_evidence_grid(fm, scales, count, seed=26, first_index=0, distributed=True, groups=None):
     """``scan_evidence`` at every frozen scale of ``scales`` (log10 Lambda) in ONE launch: each prior sample is drawn once
     and evaluated at all scales (``gf_scan_evidence_grid``; ``scripts/sens.py:199-201, 232-294`` runs one MultiNest job per
-    scale).  The model must not sample the scale (``args.fixed_scale``).  Returns ``lnZ[len(scales)]``."""
+    scale).  The model must not sample the scale (``args.fixed_scale``).  Returns ``lnZ[len(scales)]``.
+
+    With ``groups=R`` (a power of two in [2, 32]) the same launch also splits the samples into R fixed groups, sample i (global
+    index) in group i mod R (``gf_scan_evidence_grid_groups``), and returns ``(lnZ[ns], loo[R, ns])``: ``loo[r]`` is lnZ
+    without group r, the input of ``sens.evidence_error``.  lnZ equals the ungrouped result up to rounding."""
+    R = _check_groups(groups, count)
     torch = _lib.torch_cuda()
     dist = _dist() if distributed else None
     rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
     start, n = shard_range(count, rank, world, first_index)
     sc = torch.as_tensor(np.ascontiguousarray(scales, dtype=np.float64)).cuda()
     ns = int(sc.numel())
-    lse = torch.empty((ns, 2), dtype=torch.float64, device='cuda')
-    lse[:, 0] = -np.inf
-    lse[:, 1] = 0.0
+    lse = torch.empty((ns, 2) if R is None else (ns, R, 2), dtype=torch.float64, device='cuda')
+    lse[..., 0] = -np.inf
+    lse[..., 1] = 0.0
     lib = _lib.load()
-    nbytes = int(lib.gf_scan_evidence_grid_workspace(ns))
-    work = torch.empty(max(nbytes, 1), dtype=torch.uint8, device='cuda')
     cfg = _lib.ScanConfig(seed=int(seed), first_index=int(start), count=int(n), nb=0)
-    _lib.check(lib.gf_scan_evidence_grid(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, _lib.ptr(lse), _lib.ptr(work), nbytes, _lib.stream_ptr(torch)))
+    if R is None:
+        nbytes = int(lib.gf_scan_evidence_grid_workspace(ns))
+        work = torch.empty(max(nbytes, 1), dtype=torch.uint8, device='cuda')
+        _lib.check(lib.gf_scan_evidence_grid(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, _lib.ptr(lse), _lib.ptr(work), nbytes, _lib.stream_ptr(torch)))
+    else:
+        nbytes = int(lib.gf_scan_evidence_grid_groups_workspace(ns, R))
+        _lib.check(lib.gf_scan_evidence_grid_groups(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, R, _lib.ptr(lse), _lib.ptr(_workspace(torch, nbytes)), nbytes,
+                                                    _lib.stream_ptr(torch)))
     if dist and world > 1:
         lse = _lse_allreduce(dist, lse)
-    return _lnz(lse.cpu().numpy(), count)
+    if R is None:
+        return _lnz(lse.cpu().numpy(), count)
+    return _group_lnz(lse.cpu().numpy(), count, first_index)
+
+
+def _check_groups(groups, count):
+    """``groups`` of a grouped evidence call as an int (None stays None); ValueError unless it is a power of two in [2, 32] and
+    ``count`` holds at least one sample per group."""
+    if groups is None:
+        return None
+    R = int(groups)
+    if R != groups or R < 2 or R > _lib.GF_EVIDENCE_MAX_GROUPS or R & (R - 1):
+        raise ValueError('groups = %r: a power of two in [2, %d] is required' % (groups, _lib.GF_EVIDENCE_MAX_GROUPS))
+    if int(count) < R:
+        raise ValueError('%d samples for %d groups: every group needs at least one sample' % (int(count), R))
+    return R
+
+
+def group_sizes(count, groups, first_index=0):
+    """n_r: the number of global sample indices i in [first_index, first_index + count) with i mod groups = r, for r < groups."""
+    r = np.arange(int(groups))
+    below = lambda b: (b - r + groups - 1) // groups   # noqa: E731  (# of i in [0, b) with i = r mod groups)
+    return below(int(first_index) + int(count)) - below(int(first_index))
+
+
+def _group_lnz(h, count, first_index=0):
+    """(lnZ [...], leave-one-group-out lnZ [..., R, ns]) of grouped (max, sum) pairs h[..., ns, R, 2] over the global index
+    range [first_index, first_index + count): lnZ = LSE over all groups - ln N, lnZ_(-r) = LSE over the groups != r -
+    ln(N - n_r).  O(R) per (..., scale): the group weights relative to the largest one are summed from both ends, and the
+    weight without group r joins the prefix before r with the suffix after it -- no subtraction, so a group holding nearly all
+    the weight does not cancel the others away.  Where a group lies more than 700 e-folds below the largest (its relative
+    weight would be subnormal or zero) the row takes np.logaddexp.accumulate instead."""
+    R = h.shape[-2]
+    n_r = group_sizes(count, R, first_index)
+    with np.errstate(divide='ignore'):
+        lw = np.where(h[..., 1] > 0, h[..., 0] + np.log(np.where(h[..., 1] > 0, h[..., 1], 1.0)), -np.inf)   # [..., ns, R]
+    top = lw.max(axis=-1, keepdims=True)
+    ref = np.where(np.isfinite(top), top, 0.0)
+    w = np.exp(lw - ref)
+    zero = np.zeros(w.shape[:-1] + (1,))
+    pre = np.concatenate([zero, np.cumsum(w, axis=-1)[..., :-1]], axis=-1)                  # groups before r
+    suf = np.concatenate([np.cumsum(w[..., ::-1], axis=-1)[..., -2::-1], zero], axis=-1)    # groups after r
+    with np.errstate(divide='ignore'):
+        rest = np.log(pre + suf) + ref
+        tot = np.log(w.sum(axis=-1)) + ref[..., 0]
+    deep = np.any(np.isfinite(lw) & (lw - ref < -700.0), axis=-1)
+    if deep.any():
+        d = lw[deep]
+        acc = np.logaddexp.accumulate(d, axis=-1)
+        back = np.flip(np.logaddexp.accumulate(np.flip(d, axis=-1), axis=-1), axis=-1)
+        none = np.full(d.shape[:-1] + (1,), -np.inf)
+        rest[deep] = np.logaddexp(np.concatenate([none, acc[..., :-1]], axis=-1), np.concatenate([back[..., 1:], none], axis=-1))
+        tot[deep] = acc[..., -1]
+    with np.errstate(divide='ignore'):
+        return tot - np.log(count), np.moveaxis(rest - np.log(count - n_r), -1, -2)
 
 
 def source_rows(sources, injected):
@@ -287,18 +351,27 @@ def source_rows(sources, injected):
     return np.ascontiguousarray(src), inj
 
 
-def _sources_launch(lib, fm, cfg, sc, ns, src, inj, lse, stream):
+def _sources_launch(lib, fm, cfg, sc, ns, src, inj, lse, stream, groups=None):
     """Enqueue ``gf_scan_evidence_sources`` for ``src`` / ``inj`` (any length: split into calls of at most ``GF_SRC_MAX``)
-    into ``lse`` [nsrc, ns, 2] (a contiguous CUDA tensor)."""
+    into ``lse`` [nsrc, ns, 2] (a contiguous CUDA tensor).  With ``groups=R``: ``gf_scan_evidence_sources_groups`` into ``lse``
+    [nsrc, ns, R, 2], in calls of at most ``min(GF_SRC_MAX, GF_EVS_MAX_UNITS / R)`` sources."""
     torch = _lib.torch_cuda()
-    for j0 in range(0, src.shape[0], _lib.GF_SRC_MAX):
-        s, i = src[j0:j0 + _lib.GF_SRC_MAX], inj[j0:j0 + _lib.GF_SRC_MAX]
+    R = 1 if groups is None else int(groups)
+    per = min(_lib.GF_SRC_MAX, _lib.GF_EVS_MAX_UNITS // R)
+    for j0 in range(0, src.shape[0], per):
+        s, i = src[j0:j0 + per], inj[j0:j0 + per]
         n = s.shape[0]
-        nbytes = int(lib.gf_scan_evidence_sources_workspace(ns, n))
-        work = _workspace(torch, nbytes)
-        _lib.check(lib.gf_scan_evidence_sources(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, s.ctypes.data_as(C.c_void_p),
-                                                i.ctypes.data_as(C.c_void_p), n, C.c_void_p(lse.data_ptr() + 16 * ns * j0),
-                                                _lib.ptr(work), nbytes, stream))
+        out = C.c_void_p(lse.data_ptr() + 16 * ns * R * j0)
+        if groups is None:
+            nbytes = int(lib.gf_scan_evidence_sources_workspace(ns, n))
+            work = _workspace(torch, nbytes)
+            _lib.check(lib.gf_scan_evidence_sources(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, s.ctypes.data_as(C.c_void_p),
+                                                    i.ctypes.data_as(C.c_void_p), n, out, _lib.ptr(work), nbytes, stream))
+        else:
+            nbytes = int(lib.gf_scan_evidence_sources_groups_workspace(ns, n, R))
+            work = _workspace(torch, nbytes)
+            _lib.check(lib.gf_scan_evidence_sources_groups(fm.ref, C.byref(cfg), _lib.ptr(sc), ns, s.ctypes.data_as(C.c_void_p),
+                                                           i.ctypes.data_as(C.c_void_p), n, R, out, _lib.ptr(work), nbytes, stream))
 
 
 _WORK = {}
@@ -330,28 +403,34 @@ def _lnz(h, count):
         return np.where(h[..., 1] > 0, h[..., 0] + np.log(h[..., 1]) - np.log(count), -np.inf)
 
 
-def scan_evidence_sources(fm, scales, sources, injected, count, seed=26, first_index=0, distributed=True):
+def scan_evidence_sources(fm, scales, sources, injected, count, seed=26, first_index=0, distributed=True, groups=None):
     """``scan_evidence_grid`` for many source compositions at once: ``lnZ[nsrc, len(scales)]``, row j the evidence grid of a
     model whose source is ``sources[j]`` and whose injected composition is ``injected[j]`` (or the one shared ``injected``
     [3]).  ONE launch per ``GF_SRC_MAX`` sources (``gf_scan_evidence_sources``): every prior sample is drawn and run through
     the eigen stage once per scale, then scored for every source.  The model's own source and injected composition are
     ignored; it must not sample the scale or the source and must have the Gaussian likelihood.  Sharded over ranks and merged
-    like ``scan_evidence_grid``."""
+    like ``scan_evidence_grid``.
+
+    With ``groups=R`` returns ``(lnZ[nsrc, ns], loo[nsrc, R, ns])`` as ``scan_evidence_grid`` does (``gf_scan_evidence_sources_groups``;
+    one launch per ``min(256, 4096 / R)`` sources)."""
     src, inj = source_rows(sources, injected)
+    R = _check_groups(groups, count)
     torch = _lib.torch_cuda()
     dist = _dist() if distributed else None
     rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
     start, n = shard_range(count, rank, world, first_index)
     sc = torch.as_tensor(np.ascontiguousarray(scales, dtype=np.float64).ravel()).cuda()
     ns = int(sc.numel())
-    lse = torch.empty((src.shape[0], ns, 2), dtype=torch.float64, device='cuda')
+    lse = torch.empty((src.shape[0], ns, 2) if R is None else (src.shape[0], ns, R, 2), dtype=torch.float64, device='cuda')
     lse[..., 0] = -np.inf
     lse[..., 1] = 0.0
     cfg = _lib.ScanConfig(seed=int(seed), first_index=int(start), count=int(n), nb=0)
-    _sources_launch(_lib.load(), fm, cfg, sc, ns, src, inj, lse, _lib.stream_ptr(torch))
+    _sources_launch(_lib.load(), fm, cfg, sc, ns, src, inj, lse, _lib.stream_ptr(torch), groups=R)
     if dist and world > 1:
         lse = _lse_allreduce(dist, lse)
-    return _lnz(lse.cpu().numpy(), count)
+    if R is None:
+        return _lnz(lse.cpu().numpy(), count)
+    return _group_lnz(lse.cpu().numpy(), count, first_index)
 
 
 # defaults of the profile optimiser, from the host-harness study recorded in DESIGN.md (K3c)

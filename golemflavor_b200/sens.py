@@ -19,11 +19,11 @@ from . import model as _model
 from .enums import ParamTag, Texture
 from .mcmc import DeviceEnsembleSampler
 from .param import Param, ParamSet
-from .scan import (DEFAULT_BINNING, PROFILE_NSTARTS, _dist, _lnz, _lse_allreduce, _profile_launch, _profile_sources_launch, _sources_launch,
-                   _workspace, shard_range, sm_paramset, source_rows)
+from .scan import (DEFAULT_BINNING, PROFILE_NSTARTS, _check_groups, _dist, _group_lnz, _lnz, _lse_allreduce, _profile_launch, _profile_sources_launch,
+                   _sources_launch, _workspace, shard_range, sm_paramset, source_rows)
 
-__all__ = ['scale_grid', 'sweep_paramset', 'sweep', 'evidence_grid', 'evidence_source_grid', 'profile_grid', 'profile_source_grid', 'get_limit',
-           'limits', 'limit_table', 'BAYES_K', 'FREQ_CL']
+__all__ = ['scale_grid', 'sweep_paramset', 'sweep', 'evidence_grid', 'evidence_source_grid', 'evidence_error', 'profile_grid', 'profile_source_grid',
+           'get_limit', 'limits', 'limit_table', 'BAYES_K', 'FREQ_CL']
 
 
 def scale_grid(dimension, segments):
@@ -134,7 +134,8 @@ def sweep(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, sour
 
 
 def evidence_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, source_ratio=(1, 2, 0),
-                  injected_ratio=(1, 1, 1), smearing=0.02, samples=1_000_000, seed=26, binning=DEFAULT_BINNING, return_maxllh=False):
+                  injected_ratio=(1, 1, 1), smearing=0.02, samples=1_000_000, seed=26, binning=DEFAULT_BINNING, return_maxllh=False,
+                  groups=None):
     """Monte-Carlo evidence per (dimension, scale) grid point (``scripts/sens.py:289-294`` stores
     ``(scale, lnZ)`` per point): the six SM nuisance parameters are drawn from their priors, the scale is
     frozen at the grid value, ``lnZ = ln mean(L)``.  Returns ``{dimension: array[segments, 2]}`` like the
@@ -142,10 +143,17 @@ def evidence_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.O
     ln L among the samples); Bayes factors against the null point (scale -100) and the limit follow with
     ``get_limit`` (``plot.py:149-213``).
 
-    ONE launch per dimension (``gf_scan_evidence_grid``): every prior sample is drawn once, the scale-independent part
-    of the physics is built once, and the sample is evaluated at all scales of the grid; samples are sharded over the
-    ranks of the process group and the per-scale (max, sum-exp) pairs are merged with two all-reduces at the end."""
+    With ``groups=R`` (a power of two in [2, 32], at most ``samples``) the same launches split the samples into R fixed groups,
+    sample i in group i mod R, and the leave-one-group-out curves ``{dimension: array[R, segments, 2]}`` of (scale, lnZ without
+    group r) are returned last: ``evidence_error`` gives the Monte-Carlo error of every lnZ from them, ``limit_table(..., loo=)``
+    the error of the limit.  lnZ itself equals the ungrouped result up to rounding.
+
+    ONE launch per dimension (``gf_scan_evidence_grid``, ``gf_scan_evidence_grid_groups`` with groups): every prior sample is
+    drawn once, the scale-independent part of the physics is built once, and the sample is evaluated at all scales of the grid;
+    samples are sharded over the ranks of the process group and the per-scale (max, sum-exp) pairs are merged with two
+    all-reduces at the end."""
     import ctypes as C
+    R = _check_groups(groups, samples)
     torch = _lib.torch_cuda()
     dist = _dist()
     rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
@@ -156,27 +164,39 @@ def evidence_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.O
     nsc = [len(g) for g in grids]
     offs = np.concatenate([[0], np.cumsum(nsc)])
     scales = torch.as_tensor(np.concatenate(grids)).cuda()
-    lse = torch.empty((int(offs[-1]), 2), dtype=torch.float64, device='cuda')
-    lse[:, 0] = -np.inf
-    lse[:, 1] = 0.0
+    lse = torch.empty((int(offs[-1]), 2) if R is None else (int(offs[-1]), R, 2), dtype=torch.float64, device='cuda')
+    lse[..., 0] = -np.inf
+    lse[..., 1] = 0.0
     start, n = shard_range(samples, rank, world)
     cfg = _lib.ScanConfig(seed=int(seed), first_index=int(start), count=int(n), nb=0)
     lib, stream = _lib.load(), _lib.stream_ptr(torch)
-    work_bytes = int(lib.gf_scan_evidence_grid_workspace(max(nsc)))
+    if R is None:
+        work_bytes = int(lib.gf_scan_evidence_grid_workspace(max(nsc)))
+    else:
+        work_bytes = int(lib.gf_scan_evidence_grid_groups_workspace(max(nsc), R))
     work = _workspace(torch, work_bytes)
     for k, dim in enumerate(dims):
         fm = _grid_model(dim, texture, src, inj, smearing, binning)
-        _lib.check(lib.gf_scan_evidence_grid(fm.ref, C.byref(cfg), C.c_void_p(scales.data_ptr() + 8 * int(offs[k])), nsc[k],
-                                             C.c_void_p(lse.data_ptr() + 16 * int(offs[k])), _lib.ptr(work), work_bytes, stream))
+        sc, out = C.c_void_p(scales.data_ptr() + 8 * int(offs[k])), C.c_void_p(lse.data_ptr() + 16 * (R or 1) * int(offs[k]))
+        if R is None:
+            _lib.check(lib.gf_scan_evidence_grid(fm.ref, C.byref(cfg), sc, nsc[k], out, _lib.ptr(work), work_bytes, stream))
+        else:
+            _lib.check(lib.gf_scan_evidence_grid_groups(fm.ref, C.byref(cfg), sc, nsc[k], R, out, _lib.ptr(work), work_bytes, stream))
     if dist and world > 1:
         lse = _lse_allreduce(dist, lse)
     h = lse.cpu().numpy()
-    lnz = _lnz(h, samples)
     allsc = np.concatenate(grids)
+    if R is None:
+        lnz, maxllh = _lnz(h, samples), h[:, 0]
+    else:
+        (lnz, loo), maxllh = _group_lnz(h, samples), h[..., 0].max(axis=-1)
     ev = {d: np.column_stack([allsc[offs[k]:offs[k + 1]], lnz[offs[k]:offs[k + 1]]]) for k, d in enumerate(dims)}
+    out = (ev,)
     if return_maxllh:
-        return ev, {d: np.column_stack([allsc[offs[k]:offs[k + 1]], h[offs[k]:offs[k + 1], 0]]) for k, d in enumerate(dims)}
-    return ev
+        out += ({d: np.column_stack([allsc[offs[k]:offs[k + 1]], maxllh[offs[k]:offs[k + 1]]]) for k, d in enumerate(dims)},)
+    if R is not None:
+        out += ({d: np.stack([np.broadcast_to(grids[k], (R, nsc[k])), loo[:, offs[k]:offs[k + 1]]], axis=-1) for k, d in enumerate(dims)},)
+    return out[0] if len(out) == 1 else out
 
 
 def _grid_model(dim, texture, src, inj, smearing, binning):
@@ -188,7 +208,7 @@ def _grid_model(dim, texture, src, inj, smearing, binning):
 
 
 def evidence_source_grid(sources, dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, injected_ratio=(1, 1, 1),
-                         smearing=0.02, samples=1_000_000, seed=26, binning=DEFAULT_BINNING):
+                         smearing=0.02, samples=1_000_000, seed=26, binning=DEFAULT_BINNING, groups=None):
     """``evidence_grid`` for every source composition of ``sources`` ([nsrc, 3], or one [3]) at once: the reference's
     submitter runs ``scripts/sens.py`` once per (dimension, texture, source composition, Lambda segment), 30 compositions per
     texture (``submitter/sens_dag.py:8-16, 38-61, 76-95``).  ``injected_ratio`` is one composition shared by all sources or
@@ -196,18 +216,22 @@ def evidence_source_grid(sources, dimensions=(3, 4, 5, 6, 7, 8), segments=100, t
     ``evidence_grid(source_ratio=sources[j], injected_ratio=...)[d]`` (the null point -100 and the same scale grid) and the
     same samples.  ``limit_table`` turns the result into limits.
 
-    ONE launch per dimension (``gf_scan_evidence_sources``; per 256 sources beyond that): the eigen stage of each prior sample
-    runs once per scale, and every source is then scored from its transition sums.  The model of a dimension is built like
-    ``evidence_grid``'s (``_grid_model``); samples are sharded over the ranks of the process group and merged with two
-    all-reduces."""
+    With ``groups=R`` also the leave-one-group-out curves ``{dimension: array[nsrc, R, segments, 2]}`` (see ``evidence_grid``):
+    ``evidence_error`` and ``limit_table(ev, loo=...)`` turn them into errors of lnZ and of the limits.
+
+    ONE launch per dimension (``gf_scan_evidence_sources``; per 256 sources beyond that, and with groups per ``min(256, 4096 / R)``):
+    the eigen stage of each prior sample runs once per scale, and every source is then scored from its transition sums.  The
+    model of a dimension is built like ``evidence_grid``'s (``_grid_model``); samples are sharded over the ranks of the
+    process group and merged with two all-reduces."""
     src, inj = source_rows(sources, injected_ratio)
+    R = _check_groups(groups, samples)
     torch = _lib.torch_cuda()
     dist = _dist()
     rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
     dims = [int(d) for d in dimensions]
     grids = [scale_grid(d, segments) for d in dims]
     nsc = len(grids[0])
-    lse = torch.empty((len(dims), src.shape[0], nsc, 2), dtype=torch.float64, device='cuda')
+    lse = torch.empty((len(dims), src.shape[0], nsc, 2) if R is None else (len(dims), src.shape[0], nsc, R, 2), dtype=torch.float64, device='cuda')
     lse[..., 0] = -np.inf
     lse[..., 1] = 0.0
     start, n = shard_range(samples, rank, world)
@@ -217,11 +241,49 @@ def evidence_source_grid(sources, dimensions=(3, 4, 5, 6, 7, 8), segments=100, t
     # the model's own source and injected composition are ignored by the kernel: the first row stands in
     for k, dim in enumerate(dims):
         fm = _grid_model(dim, texture, src[0], inj[0], smearing, binning)
-        _sources_launch(lib, fm, cfg, scales[k], nsc, src, inj, lse[k], stream)
+        _sources_launch(lib, fm, cfg, scales[k], nsc, src, inj, lse[k], stream, groups=R)
     if dist and world > 1:
         lse = _lse_allreduce(dist, lse)
-    lnz = _lnz(lse.cpu().numpy(), samples)
-    return {d: np.stack([np.broadcast_to(grids[k], lnz[k].shape), lnz[k]], axis=-1) for k, d in enumerate(dims)}
+    if R is None:
+        lnz = _lnz(lse.cpu().numpy(), samples)
+    else:
+        lnz, loo = _group_lnz(lse.cpu().numpy(), samples)
+    ev = {d: np.stack([np.broadcast_to(grids[k], lnz[k].shape), lnz[k]], axis=-1) for k, d in enumerate(dims)}
+    if R is None:
+        return ev
+    return ev, {d: np.stack([np.broadcast_to(grids[k], loo[k].shape), loo[k]], axis=-1) for k, d in enumerate(dims)}
+
+
+def _jackknife_sigma(full, loo):
+    """Delete-one-group jackknife error of the estimates ``full`` [...] from their leave-one-out values ``loo`` [..., R]:
+    sqrt((R - 1) / R * sum_r (loo_r - mean_r loo_r)^2).  NaN where ``full`` is not finite; +inf where it is but some
+    leave-one-out value is not (all the information sits in the groups that were left out)."""
+    full, loo = np.asarray(full, dtype=np.float64), np.asarray(loo, dtype=np.float64)
+    R = loo.shape[-1]
+    if R == 0:                                                   # no leave-one-out values (an empty table): nothing to estimate
+        return np.full(full.shape, np.nan)
+    ok = np.all(np.isfinite(loo), axis=-1)
+    with np.errstate(invalid='ignore'):
+        d = loo - loo.mean(axis=-1, keepdims=True)
+        sigma = np.sqrt((R - 1) / R * np.sum(d * d, axis=-1))
+    return np.where(~np.isfinite(full), np.nan, np.where(ok, sigma, np.inf))
+
+
+def evidence_error(evidence, loo):
+    """Monte-Carlo standard error of every lnZ of a grouped ``evidence_grid`` / ``evidence_source_grid`` result: the
+    delete-one-group jackknife sigma = sqrt((R - 1) / R * sum_r (lnZ_(-r) - mean_r lnZ_(-r))^2) over the R leave-one-group-out
+    curves.  ``evidence`` ``{d: [segments, 2]}`` with ``loo`` ``{d: [R, segments, 2]}``, or ``{d: [nsrc, segments, 2]}`` with
+    ``{d: [nsrc, R, segments, 2]}``; returns ``{d: [segments]}`` or ``{d: [nsrc, segments]}``.  sigma is NaN where lnZ is -inf
+    (no sample carried weight) and +inf where lnZ is finite but some lnZ_(-r) is -inf (all the weight sits in one group)."""
+    if set(loo) != set(evidence):
+        raise ValueError('evidence_error: the leave-one-out curves have dimensions %s, the evidence %s' % (sorted(loo), sorted(evidence)))
+    out = {}
+    for d, ev in evidence.items():
+        ev, lo = np.asarray(ev, dtype=np.float64), np.asarray(loo[d], dtype=np.float64)
+        if lo.ndim != ev.ndim + 1 or lo.shape[:-3] != ev.shape[:-2] or lo.shape[-2:] != ev.shape[-2:]:
+            raise ValueError('evidence_error: dimension %s: leave-one-out curves of shape %s do not match the evidence %s' % (d, lo.shape, ev.shape))
+        out[d] = _jackknife_sigma(ev[..., 1], np.moveaxis(lo[..., 1], -2, -1))
+    return out
 
 
 def profile_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, source_ratio=(1, 2, 0),
@@ -389,30 +451,56 @@ def limits(evidence, **kwargs):
     return {d: get_limit(ev[:, 0], ev[:, 1], **kwargs) for d, ev in evidence.items()}
 
 
-def limit_table(evidence_by_source, **kwargs):
+def limit_table(evidence_by_source, loo=None, **kwargs):
     """``get_limit`` for every (dimension, source) of an ``evidence_source_grid`` result -- or of any
     ``{dimension: array[nsrc, segments, 2]}`` of (scale, statistic) curves, e.g. of ``profile_source_grid`` with
     ``args=Namespace(stat_method=StatCateg.FREQUENTIST)``: the tabulation of the reference's sensitivities
     (``plot.plot_table_sens``).  ``kwargs`` go to ``get_limit`` unchanged.  Returns ``(limits[ndims, nsrc],
     discovered[ndims, nsrc])`` with the dimensions in the dict's order: a limit is NaN where ``get_limit`` returns None or
-    raises 'Discovered LV!', and ``discovered`` is True exactly where it raises 'Discovered LV!'."""
+    raises 'Discovered LV!', and ``discovered`` is True exactly where it raises 'Discovered LV!'.
+
+    With ``loo``, the leave-one-group-out curves ``{dimension: array[nsrc, R, segments, 2]}`` of a grouped
+    ``evidence_source_grid`` (for one ``evidence_grid(..., groups=R)`` result wrap both: ``limit_table({d: ev[d][None] for d in
+    ev}, loo={d: loo[d][None] for d in loo})``), every leave-one-out curve gets its limit L_(-r) the same way, and the
+    return is ``(limits, discovered, limit_err, n_undefined)``: ``limit_err[ndims, nsrc]`` is the jackknife error
+    sqrt((R - 1) / R * sum_r (L_(-r) - mean_r L_(-r))^2) of the limit.  All scales share the samples, so it accounts for the
+    correlation between the points of a curve.  It is NaN where the limit is NaN, +inf where the limit is defined but some L_(-r)
+    is not, and ``n_undefined[ndims, nsrc]`` counts the r whose L_(-r) is not defined (no limit or 'Discovered LV!').
+    ``get_limit`` reads the crossing off 1000 spline points, so limits are quantised to that resolution: an error of 0 means
+    that the leave-one-out limits fall on the same spline point, not that the limit is exact."""
     dims = list(evidence_by_source)
     nsrc = {len(evidence_by_source[d]) for d in dims}
     if len(nsrc) > 1:
         raise ValueError('limit_table: the dimensions have different numbers of sources: %s' % sorted(nsrc))
     nsrc = nsrc.pop() if nsrc else 0
-    lim = np.full((len(dims), nsrc), np.nan)
+    R = 0
+    if loo is not None:
+        if set(loo) != set(dims):
+            raise ValueError('limit_table: the leave-one-out curves have dimensions %s, the evidence %s' % (sorted(loo), sorted(dims)))
+        R = np.shape(loo[dims[0]])[1] if dims and np.ndim(loo[dims[0]]) == 4 else 0
+        for d in dims:
+            ev_shape, lo_shape = np.shape(evidence_by_source[d]), np.shape(loo[d])
+            if len(lo_shape) != 4 or lo_shape[0] != ev_shape[0] or lo_shape[1] != R or R < 2 or lo_shape[2:] != tuple(ev_shape[1:]):
+                raise ValueError('limit_table: dimension %s: leave-one-out curves of shape %s do not match the evidence %s (expected [%d, R >= 2, %s])'
+                                 % (d, lo_shape, ev_shape, ev_shape[0], ', '.join(map(str, ev_shape[1:]))))
+    # curve 0 of a (dimension, source) is its evidence, curves 1 .. R its leave-one-out curves
+    lim = np.full((len(dims), nsrc, 1 + R), np.nan)
     disc = np.zeros((len(dims), nsrc), dtype=bool)
     for i, d in enumerate(dims):
         for j, ev in enumerate(evidence_by_source[d]):
-            ev = np.asarray(ev, dtype=np.float64)
-            try:
-                v = get_limit(ev[:, 0], ev[:, 1], **kwargs)
-            except AssertionError as e:
-                if str(e) != 'Discovered LV!':
-                    raise
-                disc[i, j] = True
-                continue
-            if v is not None:
-                lim[i, j] = v
-    return lim, disc
+            curves = [ev] if loo is None else [ev] + list(loo[d][j])
+            for c, curve in enumerate(curves):
+                curve = np.asarray(curve, dtype=np.float64)
+                try:
+                    v = get_limit(curve[:, 0], curve[:, 1], **kwargs)
+                except AssertionError as e:
+                    if str(e) != 'Discovered LV!':
+                        raise
+                    if c == 0:
+                        disc[i, j] = True
+                    continue
+                if v is not None:
+                    lim[i, j, c] = v
+    if loo is None:
+        return lim[..., 0], disc
+    return lim[..., 0], disc, _jackknife_sigma(lim[..., 0], lim[..., 1:]), np.sum(np.isnan(lim[..., 1:]), axis=-1)

@@ -232,6 +232,24 @@ int gf_scan_evidence_sources(const gf_model* model, const gf_scan_config* cfg, c
                              const double* sources /*HOST [nsrc][3]*/, const double* injected /*HOST [nsrc][3]*/, int32_t nsrc,
                              double* d_lse /*[nsrc][nscales][2]*/, void* d_work, uint64_t work_bytes, void* stream);
 /*
+ * Grouped evidence grids: the Monte-Carlo error of lnZ by a delete-one-group jackknife.  The samples are split into `groups`
+ * fixed groups, a power of two in [2, 32]: sample i (global Philox index cfg->first_index + j) is in group i mod groups, so the
+ * grouping does not depend on the launch geometry or on how the index range is sharded.  d_lse gains a group axis and
+ * accumulates (max ln L, sum exp) per (scale, group) with the rules of the ungrouped calls (NaN and -inf carry no weight;
+ * initialise to {-inf, 0}; the values already there are merged).  Merging the groups gives the ungrouped result up to
+ * rounding.  Same launch count as the ungrouped calls, one per call.  GF_ERR_ARG, with nothing enqueued, for everything the
+ * ungrouped call refuses, and for `groups` not a power of two in [2, 32], a workspace smaller than the `_workspace` size, and
+ * (source grid) nsrc * groups > 4096: one launch takes at most 4096 / groups sources (all 256 up to 16 groups, 128 at 32).
+ */
+uint64_t gf_scan_evidence_grid_groups_workspace(int32_t nscales, int32_t groups);
+int gf_scan_evidence_grid_groups(const gf_model* model, const gf_scan_config* cfg, const double* d_scales /*[nscales]*/, int32_t nscales,
+                                 int32_t groups, double* d_lse /*[nscales][groups][2]*/, void* d_work, uint64_t work_bytes, void* stream);
+uint64_t gf_scan_evidence_sources_groups_workspace(int32_t nscales, int32_t nsrc, int32_t groups);
+int gf_scan_evidence_sources_groups(const gf_model* model, const gf_scan_config* cfg, const double* d_scales /*[nscales]*/, int32_t nscales,
+                                    const double* sources /*HOST [nsrc][3]*/, const double* injected /*HOST [nsrc][3]*/, int32_t nsrc,
+                                    int32_t groups, double* d_lse /*[nsrc][nscales][groups][2]*/, void* d_work, uint64_t work_bytes,
+                                    void* stream);
+/*
  * Profile likelihood on the same grid: the frequentist statistic of scripts/sens.py (StatCateg.FREQUENTIST, whose value the
  * reference takes from GolemFit's profiled fit, gf.get_llh_freq / Likelihood.GF_FREQ).  For each frozen scale
  * d_scales[s] = log10(Lambda_s) of a model that does not sample the scale (col_scale = -1), d_best[s] = the maximum of ln_prob
