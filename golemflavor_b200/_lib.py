@@ -123,6 +123,8 @@ _SIGNATURES = {
     'gf_hist_smooth': (C.c_int, [_P, C.c_int32, C.c_uint64, _P, C.c_int32, _P, _P, _P]),
     'gf_coverage_mask_f64': (C.c_int, [_P, C.c_int64, C.c_double, _P, C.POINTER(C.c_double), C.POINTER(C.c_uint64), _P]),
     'gf_ensemble_run': (C.c_int, [C.POINTER(Model), C.POINTER(EnsembleConfig), _P, _P, _P, _P, _P, _P]),
+    'gf_autocorr_time_workspace': (C.c_uint64, [C.c_int64, C.c_int32, C.c_int64, C.c_int32]),
+    'gf_autocorr_time': (C.c_int, [_P, C.c_int64, C.c_int32, C.c_int64, C.c_int32, C.c_double, _P, _P, _P, C.c_uint64, _P]),
     'gf_selftest_math': (C.c_int, [_P, C.c_int64, _P, _P, _P]),
     'gf_selftest_trig': (C.c_int, [_P, C.c_int64, _P, _P, _P, _P]),
     'gf_selftest_log': (C.c_int, [_P, C.c_int64, _P, _P]),

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB_DIR = os.path.join(HERE, 'lib')
 LIB_PATH = os.path.join(LIB_DIR, 'libgolemflavor_b200.so')
-SOURCES = ['gf_api.cu', 'gf_lnprob.cu', 'gf_scan.cu', 'gf_ensemble.cu', 'gf_profile.cu', 'gf_sources.cu']
+SOURCES = ['gf_api.cu', 'gf_lnprob.cu', 'gf_scan.cu', 'gf_ensemble.cu', 'gf_profile.cu', 'gf_sources.cu', 'gf_autocorr.cu']
 HEADERS = ['gf_common.cuh', 'gf_model.cuh', 'gf_physics.cuh', 'gf_scan_dev.cuh', 'gf_ensemble_dev.cuh', 'gf_profile_dev.cuh', 'gf_sources_dev.cuh', 'gf_ndtri_table.h', os.path.join('..', '..', 'include', 'golemflavor_b200.h')]
 NVCC_FLAGS = ['-O3', '-std=c++17', '--threads', '4', '-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo',
               '-Xcompiler', '-fPIC', '-shared', '-Xlinker', '-soname=libgolemflavor_b200.so']

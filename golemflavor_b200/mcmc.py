@@ -8,6 +8,11 @@ a = 2) with the emcee-2 attributes the reference driver touches, and calls the l
 *vectorised* -- each half-ensemble is ONE call ``ln_prob(theta[nwalkers/2, ndim]) -> [nwalkers/2]``,
 i.e. one CUDA kernel launch.  Only the proposal bookkeeping (a few vector operations on
 ``nwalkers x ndim`` numbers) runs in NumPy; every log-posterior value comes from the GPU.
+
+The convergence diagnostic, the integrated autocorrelation time tau that ``sampler.acor`` prints, is computed where the
+chain lives: ``autocorr_time`` runs the estimator of ``integrated_time`` on a device chain for every chain and parameter
+in one call (C ABI ``gf_autocorr_time``), and ``DeviceEnsembleSampler.get_autocorr_time`` uses it.  ``integrated_time``
+stays the host reference.
 """
 
 import os
@@ -15,7 +20,8 @@ import sys
 
 import numpy as np
 
-__all__ = ['EnsembleSampler', 'DeviceEnsembleSampler', 'mcmc', 'flat_seed', 'gaussian_seed', 'save_chains', 'integrated_time']
+__all__ = ['EnsembleSampler', 'DeviceEnsembleSampler', 'mcmc', 'flat_seed', 'gaussian_seed', 'save_chains', 'integrated_time',
+           'autocorr_time']
 
 
 def _progress(iterable, total):
@@ -48,6 +54,43 @@ def integrated_time(x, c=5.0):
         m = int(np.argmax(window)) if window.any() else nsteps - 1
         tau[d] = taus[m]
     return tau
+
+
+def _autocorr_device(chain, c=5.0):
+    """(tau [C, D], window [C, D]) CUDA tensors of a contiguous float64 CUDA chain [C, W, N, D], enqueued on the current
+    stream (``gf_autocorr_time``)."""
+    from . import _lib
+    torch = _lib.torch_cuda()
+    nchains, nwalkers, nsteps, ndim = (int(v) for v in chain.shape)
+    lib = _lib.load()
+    nbytes = lib.gf_autocorr_time_workspace(nchains, nwalkers, nsteps, ndim)
+    tau = torch.empty((nchains, ndim), dtype=torch.float64, device=chain.device)
+    window = torch.empty((nchains, ndim), dtype=torch.int64, device=chain.device)
+    work = torch.empty((max(int(nbytes), 1),), dtype=torch.uint8, device=chain.device)
+    _lib.check(lib.gf_autocorr_time(_lib.ptr(chain), nchains, nwalkers, nsteps, ndim, float(c), _lib.ptr(tau), _lib.ptr(window),
+                                    _lib.ptr(work), int(nbytes), _lib.stream_ptr(torch)))
+    return tau, window
+
+
+def autocorr_time(chain, c=5.0, return_window=False):
+    """Integrated autocorrelation time of a device chain: ``integrated_time`` (same definition, same window rule) for
+    every chain and parameter in one device call.
+
+    ``chain`` is a float64 CUDA tensor ``[C, W, N, D]`` (``DeviceEnsembleSampler``'s layout: chain, walker, step,
+    parameter) or ``[W, N, D]``; it is made contiguous and processed on the current stream.  Returns tau as a NumPy array
+    ``[C, D]`` (``[D]`` for a 3-D chain), with ``return_window`` also the windows m (int64, same shape): tau = tau(m).
+    Only the lags up to the window are computed.  A walker whose values are bitwise equal contributes an autocorrelation
+    of 0, so a parameter that is constant in every walker (a frozen column) gets tau = -1 at m = 0."""
+    from . import _lib
+    torch = _lib.torch_cuda()
+    if not isinstance(chain, torch.Tensor) or not chain.is_cuda or chain.dtype != torch.float64 or chain.ndim not in (3, 4):
+        raise ValueError('autocorr_time needs a float64 CUDA tensor [C, W, N, D] or [W, N, D]')
+    one = chain.ndim == 3
+    tau, window = _autocorr_device((chain.unsqueeze(0) if one else chain).contiguous(), c=c)
+    tau, window = tau.cpu().numpy(), window.cpu().numpy()
+    if one:
+        tau, window = tau[0], window[0]
+    return (tau, window) if return_window else tau
 
 
 class EnsembleSampler(object):
@@ -224,11 +267,13 @@ class DeviceEnsembleSampler(object):
         return self.get_autocorr_time()
 
     def get_autocorr_time(self, c=5.0):
-        ch = self._cat(self._chains, (self.dim,))
-        if ch.shape[2] < 50:
+        """tau per chain and parameter (``autocorr_time`` on the device chain: the parts of several ``run_mcmc`` calls are
+        joined on the device, nothing is copied to the host but the result)."""
+        if sum(int(x.shape[2]) for x in self._chains) < 50:
             raise RuntimeError('The chain is too short to reliably estimate the autocorrelation time')
-        tau = np.array([integrated_time(np.swapaxes(x, 0, 1), c=c) for x in ch])
-        return self._squeeze(tau)
+        import torch
+        ch = self._chains[0] if len(self._chains) == 1 else torch.cat(self._chains, dim=2)
+        return self._squeeze(autocorr_time(ch, c=c))
 
     def run_mcmc(self, pos0, N, lnprob0=None, thin=1, store=True, return_tensor=False, check_nan=True):
         """Advance all chains by N steps.  pos0 [nwalkers, ndim] or [nchains, nwalkers, ndim]

@@ -17,7 +17,7 @@ import numpy as np
 from . import _lib, llh
 from . import model as _model
 from .enums import ParamTag, Texture
-from .mcmc import DeviceEnsembleSampler
+from .mcmc import DeviceEnsembleSampler, _autocorr_device
 from .param import Param, ParamSet
 from .scan import (DEFAULT_BINNING, PROFILE_NSTARTS, _check_groups, _dist, _group_lnz, _lnz, _lse_allreduce, _profile_launch, _profile_sources_launch,
                    _sources_launch, _workspace, shard_range, sm_paramset, source_rows)
@@ -70,12 +70,19 @@ def _dim_stream(torch, dim):
 
 def sweep(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, source_ratio=(1, 2, 0),
           injected_ratio=(1, 1, 1), smearing=0.02, nwalkers=60, burnin=200, nsteps=1000, seed=25,
-          binning=DEFAULT_BINNING, distributed=True):
+          binning=DEFAULT_BINNING, distributed=True, autocorr=False):
     """Run one chain per (dimension, scale) grid point.
 
     Returns a dict of arrays over all grid points (identical on every rank):
     ``dimension``, ``scale``, ``mean_lnprob`` (posterior mean of ln_prob), ``max_lnprob``,
     ``acceptance`` (mean acceptance fraction), ``mean_fr`` [n, 3] (posterior-mean measured composition).
+
+    ``autocorr=True`` adds ``tau`` [n, 6]: the integrated autocorrelation time (``mcmc.autocorr_time``, c = 5) of each grid
+    point's post-burn-in chain for the six SM nuisance parameters (the frozen scale column is left out), so that a point
+    can be checked against emcee's rule of thumb nsteps >= 50 tau.  The post-burn-in chain is then stored on the device,
+    nchains x nwalkers x nsteps x 7 doubles per dimension (336 MB at 100 chains x 60 walkers x 1000 steps) plus the
+    estimator's workspace, and each dimension's chains go through one ``gf_autocorr_time`` call on that dimension's stream.
+    The other outputs are the same as without it.
     """
     torch = _lib.torch_cuda()
     dist = _dist() if distributed else None
@@ -83,7 +90,7 @@ def sweep(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, sour
     grid = [(int(d), float(s)) for d in dimensions for s in scale_grid(d, segments)]
     start, count = shard_range(len(grid), rank, world)
     mine = grid[start:start + count]
-    rows = torch.zeros((len(grid), 8), dtype=torch.float64, device='cuda')
+    rows = torch.zeros((len(grid), 14 if autocorr else 8), dtype=torch.float64, device='cuda')
     src = np.asarray(source_ratio, dtype=np.float64)
     inj = np.asarray(injected_ratio, dtype=np.float64)
     # one CUDA stream per dimension: the launches of different dimensions (different models, hence different
@@ -108,14 +115,15 @@ def sweep(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, sour
         stream.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(stream):
             sampler = DeviceEnsembleSampler(nwalkers, ndim, fn, nchains=nchains, seed=seed + 1000 * dim, nfree=ndim - 1,
-                                            chain0=idx[0])
+                                            chain0=idx[0], store_lnprob=not autocorr)   # tau needs the positions only
             sampler.run_mcmc(p0, burnin, store=False, return_tensor=True, check_nan=False)   # seeds lie inside the prior box
             sampler.reset()
-            pos, lnp, _ = sampler.run_mcmc(None, nsteps, store=False, return_tensor=True)
+            pos, lnp, _ = sampler.run_mcmc(None, nsteps, store=autocorr, return_tensor=True)
             # summaries from the final ensemble + the acceptance counters (no chain leaves the device)
             _, fr, _ = fn.evaluate(pos.reshape(-1, ndim), want_fr=True, want_status=True)
-        pending.append((stream, dim, idx, scales, sampler, lnp, fr, nchains))
-    for stream, dim, idx, scales, sampler, lnp, fr, nchains in pending:
+            tau = _autocorr_device(sampler._chains[0])[0] if autocorr else None
+        pending.append((stream, dim, idx, scales, sampler, lnp, fr, nchains, tau))
+    for stream, dim, idx, scales, sampler, lnp, fr, nchains, tau in pending:
         stream.synchronize()
         fr = fr.reshape(nchains, nwalkers, 3)
         acc = torch.as_tensor(np.atleast_2d(sampler.acceptance_fraction), device='cuda').reshape(nchains, nwalkers)
@@ -126,11 +134,16 @@ def sweep(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, sour
         rows[ii, 3] = lnp.max(dim=1).values
         rows[ii, 4] = acc.mean(dim=1)
         rows[ii, 5:8] = fr.mean(dim=1)
+        if autocorr:
+            rows[ii, 8:14] = tau[:, :6]
     if dist and world > 1:
         dist.all_reduce(rows, op=dist.ReduceOp.SUM)              # disjoint rows: sum == gather
     out = rows.cpu().numpy()
-    return {'dimension': out[:, 0].astype(int), 'scale': out[:, 1], 'mean_lnprob': out[:, 2], 'max_lnprob': out[:, 3],
-            'acceptance': out[:, 4], 'mean_fr': out[:, 5:8]}
+    res = {'dimension': out[:, 0].astype(int), 'scale': out[:, 1], 'mean_lnprob': out[:, 2], 'max_lnprob': out[:, 3],
+           'acceptance': out[:, 4], 'mean_fr': out[:, 5:8]}
+    if autocorr:
+        res['tau'] = out[:, 8:14]
+    return res
 
 
 def evidence_grid(dimensions=(3, 4, 5, 6, 7, 8), segments=100, texture=Texture.OET, source_ratio=(1, 2, 0),

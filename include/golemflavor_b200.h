@@ -368,6 +368,23 @@ typedef struct gf_ensemble_config {
  * [nchains][nwalkers][nsteps/thin], d_naccept [nchains][nwalkers] (ADDS accepted-move counts). */
 int gf_ensemble_run(const gf_model* model, const gf_ensemble_config* cfg, double* d_pos, double* d_lnp, double* d_chain,
                     double* d_lnp_chain, unsigned long long* d_naccept, void* stream);
+/*
+ * Integrated autocorrelation time of stored chains (emcee's get_autocorr_time, golemflavor/mcmc.py:46-49), for every chain
+ * and parameter of d_chain[nchains][nwalkers][nsteps][ndim] (gf_ensemble_run's layout).  For chain c, parameter d and
+ * walker w with y = x_w - mean(x_w): a_w(t) = sum_{i < nsteps-t} y_i y_{i+t}; rho_w(t) = a_w(t) / a_w(0) if a_w(0) > 0,
+ * else 0; acf(t) = the mean of rho_w(t) over all walkers; tau(t) = 2 sum_{s <= t} acf(s) - 1.  d_window[c][d] = m, the
+ * first t with t >= c * tau(t) (nsteps - 1 if there is none), and d_tau[c][d] = tau(m).  A walker whose values are
+ * bitwise equal contributes rho = 0, so a parameter constant in every walker gets tau = -1 at m = 0.  Lags are computed
+ * in tiles of 256 and stop at the tile holding every pair's window: 1 + 2 ceil(nsteps / 256) launches at most, no host
+ * synchronisation, no float atomics (bit-identical results; a chain's result does not depend on the other chains).
+ * d_work is scratch of at least gf_autocorr_time_workspace(...) bytes (0 for a shape the call refuses).  GF_ERR_ARG, with
+ * nothing enqueued, for: a null pointer; nchains < 1, nwalkers < 1 or nsteps < 2; ndim outside [1, GF_MAX_DIM];
+ * nchains * nwalkers > 2^31 - 1; c not finite and positive; a workspace too small.
+ */
+uint64_t gf_autocorr_time_workspace(int64_t nchains, int32_t nwalkers, int64_t nsteps, int32_t ndim);
+int gf_autocorr_time(const double* d_chain /*[nchains][nwalkers][nsteps][ndim]*/, int64_t nchains, int32_t nwalkers, int64_t nsteps,
+                     int32_t ndim, double c, double* d_tau /*[nchains][ndim]*/, int64_t* d_window /*[nchains][ndim]*/, void* d_work,
+                     uint64_t work_bytes, void* stream);
 
 /* ---- measurement helper ----------------------------------------------- */
 /* fp64 throughput microbenchmarks: `iters` dependent FMAs x 8 chains per thread on a full grid;
